@@ -32,6 +32,9 @@ Printed JSON (rank 0, one line):
   clocks, gpu_launches, local_shard_ms_per_step (N > 1: K2 alone, max over ranks)
 (--no-north-star: the primary workload only.)
 
+--dump-outputs DIR writes what the last timed step returned (ids, scores, counts of the primary workload) as DIR/<name>.npy.
+It is refused with --impl reference, whose steps search a query sample of their own: nothing there to compare output for output.
+
 `--impl reference` times that CPU implementation alone (numpy-only process; the reference's own dependency
 qdrant-client is not installable here, so kind="port").
 """
@@ -429,6 +432,7 @@ def run_b200(args):
     launches = _lib.kernel_launch_count() - l0
     value = nq / (ms_step / 1e3)
     counts_ok = bool((out[2] == k).all().item()) and bool(torch.equal(out[0], out_serial[0]) and torch.equal(out[2], out_serial[2]))
+    last_step = [t.cpu().numpy() for t in out] if args.dump_outputs and rank == 0 else None   # the buffers are reused by later submits
     check = verify(index, q_dev, out, k)
 
     # N > 1: the same step without the exchange + merge (K2 on the local shard only), to show what the exchange costs
@@ -786,9 +790,21 @@ def run_b200(args):
             "results_ok": bool(counts_ok and (check is None or check["ok"]) and e2e_same and (oracle_check is None or oracle_check["ok"])),
         }
         print(json.dumps(line), flush=True)
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, *last_step)
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+def dump_outputs(out_dir, ids, scores, counts):
+    """The merged (ids, scores, counts) of the last timed step, as ShardedIndex.collect hands them to a caller, so that two builds
+    can be compared output for output (the inputs are seeded).  At most 4096 x 100 results: under 5 MB in all."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "ids.npy"), ids.astype(np.float64))          # global row ids < 2**53: exact in float64
+    np.save(os.path.join(out_dir, "scores.npy"), scores.astype(np.float32))
+    np.save(os.path.join(out_dir, "counts.npy"), counts.astype(np.float64))
 
 
 def main():
@@ -807,7 +823,12 @@ def main():
                     help="primary workload only: skip the north-star series, K1, the self-join and configs[0]")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaled 100M x 1280 point (N = 2, 4)")
     ap.add_argument("--no-selfjoin", action="store_true", help="skip configs[4] (2M x 1024 self-join)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's ids / scores / counts to DIR/<name>.npy (float64 / float32 / float64); "
+                         "B200 arm only: --impl reference times a query sample of its own, not comparable output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the result of the B200 arm's timed step")
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)

@@ -128,7 +128,7 @@ def test_committed_trace_is_what_the_unmodified_reference_does_today(trace, tmp_
     assert a.keys() == b.keys() and all(np.allclose(a[k], b[k], atol=1e-6) for k in a)
 
 
-def test_oracle_embedding_half_is_pinned_to_reference_outputs(trace):
+def test_oracle_embedding_half_is_pinned_to_reference_outputs(trace, tmp_path):
     """The vectors the unmodified reference computed (core_system.py:341-349, 363, 398-408 / 442-447) and handed to
     `upsert` as python lists of floats (:608) == the oracle's restatement on the same encoder output and masks."""
     import torch
@@ -145,8 +145,9 @@ def test_oracle_embedding_half_is_pinned_to_reference_outputs(trace):
                 want = O.l2_normalize(O.global_embedding(feats)[0])
                 assert p["bbox"] == [0, 0, pil.width, pil.height] and p["area_ratio"] == 1.0
             else:                                                          # extract_embeddings, core_system.py:320-429
-                pil.convert("RGB").save("/tmp/_rvo_probe.jpg")
-                masks = det.predict("/tmp/_rvo_probe.jpg").mask
+                probe = str(tmp_path / "probe.jpg")
+                pil.convert("RGB").save(probe)
+                masks = det.predict(probe).mask
                 embs = O.extract_embeddings_reference(feats, masks)
                 kept = [j for j in range(len(masks)) if O.binarize_mask(masks[j]).sum() > 0]
                 assert len(embs) == 3 and kept == [0, 1, 3]                # the empty mask is dropped, later regions shift up
