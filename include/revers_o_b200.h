@@ -262,7 +262,10 @@ int rvo_search_topk_fused(const uint16_t* db, int64_t n_rows, int32_t d, int64_t
  *   out_count  [dev] uint64 [1]  pairs found (only the first out_cap are stored)
  *   out_overflowed [dev] int32 [1]  candidate sub-lists that overflowed (> 0: result incomplete; raise "cand_cap")
  *   workspace  [dev] rvo_selfjoin_workspace_bytes(d) bytes, 1024-B aligned
- * Multi-GPU: DB replicated, ranks take disjoint [row_lo, row_hi) ranges; no collective on the data path.
+ * Multi-GPU, two ways: (1) DB replicated, ranks take disjoint [row_lo, row_hi) ranges; no collective on the data path.
+ * (2) DB row-sharded over the devices of one process (B200VectorDB(devices=[...])): rvo_join_threshold below joins each shard
+ * with itself (triangle) and every pair of shards (rectangle, 4096-row query blocks copied to the other shard's device, each
+ * rectangle split between its two devices); no shard is moved or replicated.
  * ---------------------------------------------------------------------------------------------- */
 size_t rvo_selfjoin_workspace_bytes(int32_t d);
 int rvo_selfjoin_threshold(const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad, int64_t row_lo, int64_t row_hi,
@@ -278,6 +281,24 @@ int rvo_selfjoin_threshold_ex(const uint16_t* db, int64_t n_rows, int32_t d, int
                               float threshold, int64_t id_offset, int64_t cand_cap, int64_t* out_pairs, float* out_scores,
                               int64_t out_cap, uint64_t* out_count, int32_t* out_overflowed, void* workspace,
                               size_t workspace_bytes, void* stream);
+
+/* Threshold join between two row sets on one device, the building block of the self-join of a row-sharded collection.
+ *   qdb        [dev] tiled bf16 storage holding the query rows [q_row_lo, q_row_hi); their ids are row + q_id_offset
+ *   db         [dev] tiled bf16 storage of the n_rows target rows (a sub-range must start on a 128-row block); ids row + id_offset
+ * qdb == db with q_id_offset == id_offset: TRIANGLE, exactly rvo_selfjoin_threshold_ex(db, ..., q_row_lo, q_row_hi, ...) — pairs
+ * (i, j), i in the query rows, i < j < n_rows.  Otherwise RECTANGLE: the two row sets must be disjoint (checked by id and by
+ * address; both on the same device) and every (query, target) pair at or above the threshold is emitted.  Either way a pair
+ * is stored as (lower id, higher id) with the fp32 dot of its two stored bf16 rows, bit-identical in both modes.
+ * Unlike rvo_selfjoin_threshold[_ex] this entry APPENDS: pairs go to out_pairs / out_scores from index *out_count on, the
+ * count grows by the pairs found (only indices < out_cap are stored), and overflowed candidate sub-lists are ADDED to
+ * *out_overflowed; neither is reset, so every join of a device can share one pair buffer and one host synchronisation.
+ * cand_cap as in rvo_selfjoin_threshold_ex (>= n_rows + 4096 can never overflow).  workspace: rvo_join_workspace_bytes(d,
+ * cand_cap) bytes, 1024-B aligned. */
+size_t rvo_join_workspace_bytes(int32_t d, int64_t cand_cap);
+int rvo_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset,
+                       const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad, float threshold, int64_t id_offset,
+                       int64_t cand_cap, int64_t* out_pairs, float* out_scores, int64_t out_cap,
+                       uint64_t* out_count, int32_t* out_overflowed, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Counters for bench.py's `gpu_launches` claim: number of kernels THIS library has launched on the

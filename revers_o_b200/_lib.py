@@ -70,6 +70,10 @@ PROTOTYPES = {
     "rvo_selfjoin_threshold_ex": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_int64, C.c_int64, C.c_float,
                                             C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rvo_join_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int64]),
+    "rvo_join_threshold": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int64,
+                                     C.c_float, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_size_t, C.c_void_p]),
     "rvo_kernel_launch_count": (C.c_int64, []),
     "rvo_last_scan_ms": (C.c_float, []),
     "rvo_set_option": (C.c_int, [C.c_char_p, C.c_int64]),

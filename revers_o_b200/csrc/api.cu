@@ -17,10 +17,10 @@ extern std::atomic<long long> g_merge_trace;
 extern void* g_pool_trace;
 static std::atomic<long long> opt_select_trace{0};
 size_t selfjoin_workspace_bytes(int d, long long cand_cap);
-int launch_selfjoin(const uint16_t* db, long long n_rows, int d, long long row_lo, long long row_hi, float threshold,
-                    long long id_offset, long long cand_cap, long long* out_pairs, float* out_scores, long long out_cap,
-                    unsigned long long* out_count, int* out_overflowed, void* ws, size_t ws_bytes, int sm_count,
-                    cudaStream_t stream);
+int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi, long long q_id_offset, const uint16_t* db,
+                    long long n_rows, int d, float threshold, long long id_offset, long long cand_cap, long long* out_pairs,
+                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, bool append,
+                    void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream);
 static thread_local char g_err[512] = "";
 std::atomic<long long> g_launches{0};
 std::atomic<long long> g_chain_trace{0};
@@ -859,9 +859,57 @@ int rvo_selfjoin_threshold_ex(const uint16_t* db, int64_t n_rows, int32_t d, int
     int sm = 0;
     int rc = select_device_of(db, &sm);
     if (rc) return rc;
-    return launch_selfjoin(db, n_rows, d, row_lo, row_hi, threshold, id_offset, cand_cap, (long long*)out_pairs,
-                           out_scores, out_cap, (unsigned long long*)out_count, out_overflowed, workspace, workspace_bytes, sm,
-                           (cudaStream_t)stream);
+    return launch_selfjoin(db, row_lo, row_hi, id_offset, db, n_rows, d, threshold, id_offset, cand_cap, (long long*)out_pairs,
+                           out_scores, out_cap, (unsigned long long*)out_count, out_overflowed, false, workspace, workspace_bytes,
+                           sm, (cudaStream_t)stream);
+}
+
+size_t rvo_join_workspace_bytes(int32_t d, int64_t cand_cap) { return rvo_selfjoin_workspace_bytes_ex(d, cand_cap); }
+
+int rvo_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset, const uint16_t* db,
+                       int64_t n_rows, int32_t d, int64_t d_pad_in, float threshold, int64_t id_offset, int64_t cand_cap,
+                       int64_t* out_pairs, float* out_scores, int64_t out_cap, uint64_t* out_count, int32_t* out_overflowed,
+                       void* workspace, size_t workspace_bytes, void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(qdb && db && out_pairs && out_scores && out_count && out_overflowed && workspace, "join: null pointer");
+    RVO_REQUIRE(n_rows > 0 && n_rows < (1ll << 31) && d > 0 && q_row_lo >= 0 && q_row_lo <= q_row_hi && out_cap >= 0 &&
+                    cand_cap > 0,
+                "join: bad shape n_rows=%lld query rows [%lld,%lld)", (long long)n_rows, (long long)q_row_lo,
+                (long long)q_row_hi);
+    RVO_REQUIRE(d_pad_in == (d + kBlockK - 1) / kBlockK * kBlockK, "join: d_pad must be d rounded up to 64");
+    RVO_REQUIRE(((uintptr_t)workspace & 1023) == 0 && ((uintptr_t)db & 15) == 0 && ((uintptr_t)qdb & 15) == 0,
+                "join: alignment");
+    const bool triangle = qdb == db && q_id_offset == id_offset;
+    if (triangle) {
+        RVO_REQUIRE(q_row_hi <= n_rows, "join: query rows [%lld,%lld) outside the %lld rows of the DB", (long long)q_row_lo,
+                    (long long)q_row_hi, (long long)n_rows);
+    } else {
+        // rectangle: the two row sets must be disjoint, by id and in memory (a pair would otherwise be found twice or
+        // paired with itself)
+        RVO_REQUIRE(qdb != db, "join: qdb == db with different id offsets");
+        RVO_REQUIRE(q_id_offset + q_row_hi <= id_offset || id_offset + n_rows <= q_id_offset + q_row_lo,
+                    "join: query ids [%lld,%lld) overlap target ids [%lld,%lld)", (long long)(q_id_offset + q_row_lo),
+                    (long long)(q_id_offset + q_row_hi), (long long)id_offset, (long long)(id_offset + n_rows));
+        const size_t blk = (size_t)(d_pad_in / kTileCols) * kTileRows * kTileCols;   // bf16 elements per 128-row block
+        const uint16_t *q0 = qdb + (size_t)(q_row_lo / kTileRows) * blk,
+                       *q1 = qdb + (size_t)((q_row_hi + kTileRows - 1) / kTileRows) * blk,
+                       *t1 = db + (size_t)((n_rows + kTileRows - 1) / kTileRows) * blk;
+        RVO_REQUIRE(q_row_lo == q_row_hi || q1 <= db || t1 <= q0, "join: query rows and target rows overlap in memory");
+        int qdev = -1, tdev = -1;
+        int rc = select_device_of(qdb, nullptr);
+        if (rc) return rc;
+        RVO_CUDA(cudaGetDevice(&qdev));
+        rc = select_device_of(db, nullptr);
+        if (rc) return rc;
+        RVO_CUDA(cudaGetDevice(&tdev));
+        RVO_REQUIRE(qdev == tdev, "join: query rows on device %d, target rows on device %d", qdev, tdev);
+    }
+    int sm = 0;
+    int rc = select_device_of(db, &sm);
+    if (rc) return rc;
+    return launch_selfjoin(qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, threshold, id_offset, cand_cap,
+                           (long long*)out_pairs, out_scores, out_cap, (unsigned long long*)out_count, out_overflowed, true,
+                           workspace, workspace_bytes, sm, (cudaStream_t)stream);
 }
 
 int rvo_merge_topk(const int64_t* ids, const float* scores, const int32_t* counts, int32_t G, int32_t nq, int32_t k,

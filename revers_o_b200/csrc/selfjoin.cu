@@ -1,10 +1,17 @@
 // Near-duplicate self-join (BASELINE.json config 4; SURVEY.md §8f row 1): every stored row is a query and the
 // reference's `score_threshold` (core_system.py:663) is the only selection rule — all pairs (i, j), i < j, with
 // cos(db[i], db[j]) >= threshold.  The reference has no such feature; it reuses K2 unchanged:
-//   per block of up to 4096 query rows:  gather the rows out of the tiled DB (they ARE bf16, so the tensor-core
-//   scores are exact up to fp32 summation order) -> FILTER scan of the rows at or after the block with
-//   tau = threshold - 1e-4 -> `pairs_kernel`: fp32 re-score of every candidate with j > i, append (i, j, score).
-// Only the upper triangle is scanned (block b scans rows >= its first row), i.e. N^2 * D flops, not 2 N^2 D.
+//   per block of up to 4096 query rows:  gather the rows out of the tiled query buffer (they ARE bf16, so the tensor-core
+//   scores are exact up to fp32 summation order) -> FILTER scan of the target rows with tau = threshold - 1e-4 ->
+//   `pairs_kernel`: fp32 re-score of every candidate, append (min id, max id, score).
+// Two modes share that code:
+//   TRIANGLE  query rows and target rows are the same tiled DB: block b scans only rows >= its first row and keeps j > i,
+//             i.e. N^2 * D flops, not 2 N^2 D.
+//   RECTANGLE the query rows come from another tiled buffer on the same device (a block of another shard copied here) and
+//             are disjoint from the target rows: every target row is scanned, every candidate re-scored.  Used for the
+//             cross-shard part of the join of a row-sharded collection.
+// The re-score runs the same lanes over the same chunks in the same order in both modes and fmaf is commutative in its two
+// factors, so a pair scores bit-identically whichever of its rows is the query.
 #include "common.cuh"
 #include "scan_tc.cuh"
 #include "prep_scan_small.cuh"
@@ -13,8 +20,8 @@ namespace rvo {
 
 constexpr float kSelfJoinMargin = 1e-4f;   // fp32 summation-order slack between the MMA and the re-score
 
-// q_out[q][:] = db row (row0 + q), row-major bf16 [nq_pad][d_pad]; rows q >= nq are zero.  tau[q] = thr or +inf.
-__global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restrict__ db, long long row0, int nq, int nq_pad,
+// q_out[q][:] = qdb row (row0 + q), row-major bf16 [nq_pad][d_pad]; rows q >= nq are zero.  tau[q] = thr or +inf.
+__global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restrict__ qdb, long long row0, int nq, int nq_pad,
                                                           int d_pad, uint4* __restrict__ q_out, float* __restrict__ tau,
                                                           float thr) {
     const int q = blockIdx.x;
@@ -23,7 +30,7 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restric
     const long long r = row0 + q;
     for (int c = threadIdx.x; c < nchunk; c += blockDim.x) {
         uint4 v = make_uint4(0, 0, 0, 0);
-        if (q < nq) v = __ldg(db + (((size_t)(r >> 7) * nk + (c >> 3)) * kTileRows + (r & 127)) * 8 + (c & 7));
+        if (q < nq) v = __ldg(qdb + (((size_t)(r >> 7) * nk + (c >> 3)) * kTileRows + (r & 127)) * 8 + (c & 7));
         q_out[(size_t)q * nchunk + c] = v;
     }
     (void)nq_pad;
@@ -39,15 +46,18 @@ __device__ __forceinline__ float dot8(const uint4 a, const uint4 b, float acc) {
     return acc;
 }
 
-// grid (nq), 256 threads: candidates of query row i = row0 + q; 8 lanes per candidate.
+// grid (nq), 256 threads: candidates of query row i = row0 + q; 8 lanes per candidate.  j_floor: a candidate j is re-scored
+// when j > j_floor — the query row i in TRIANGLE mode (upper triangle, no self pair), -1 in RECTANGLE mode (every candidate).
+// Pairs are emitted as (min, max) of (i + q_id_offset, j + id_offset).
 __global__ void __launch_bounds__(256) pairs_kernel(const uint4* __restrict__ db, const uint4* __restrict__ qrows, long long row0,
                                                     long long scan_base, int d_pad, const unsigned long long* __restrict__ cand,
-                                                    const int* __restrict__ cnt, int cap, float threshold, long long id_offset,
-                                                    long long* __restrict__ out_pairs, float* __restrict__ out_scores,
-                                                    long long out_cap, unsigned long long* __restrict__ out_count,
-                                                    int* __restrict__ overflowed) {
+                                                    const int* __restrict__ cnt, int cap, float threshold, bool triangle,
+                                                    long long q_id_offset, long long id_offset, long long* __restrict__ out_pairs,
+                                                    float* __restrict__ out_scores, long long out_cap,
+                                                    unsigned long long* __restrict__ out_count, int* __restrict__ overflowed) {
     const int q = blockIdx.x;
     const long long i = row0 + q;
+    const long long j_floor = triangle ? i : -1;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
     const int g = lane >> 3, l8 = lane & 7;
     const int nchunk = d_pad >> 3, nk = d_pad / kTileCols;
@@ -63,7 +73,7 @@ __global__ void __launch_bounds__(256) pairs_kernel(const uint4* __restrict__ db
             const int e = e0 + warp * 4 + g;
             long long j = -1;
             if (e < c) j = scan_base + (long long)key_row(list[e]);
-            const bool active = j > i;  // upper triangle only (also drops the self pair)
+            const bool active = e < c && j > j_floor;
             float acc = 0.f;
             if (active) {
                 const uint4* r = db + ((size_t)(j >> 7) * nk * kTileRows + (j & 127)) * 8;
@@ -81,8 +91,9 @@ __global__ void __launch_bounds__(256) pairs_kernel(const uint4* __restrict__ db
                 if (hit) {
                     const unsigned long long at = base + __popc(bal & ((1u << lane) - 1u));
                     if ((long long)at < out_cap) {
-                        out_pairs[2 * at] = i + id_offset;
-                        out_pairs[2 * at + 1] = j + id_offset;
+                        const long long gi = i + q_id_offset, gj = j + id_offset;
+                        out_pairs[2 * at] = gi < gj ? gi : gj;
+                        out_pairs[2 * at + 1] = gi < gj ? gj : gi;
                         out_scores[at] = acc;
                     }
                 }
@@ -131,35 +142,43 @@ size_t selfjoin_workspace_bytes(int d, long long cand_cap) {
     return sp.bytes;
 }
 
-int launch_selfjoin(const uint16_t* db, long long n_rows, int d, long long row_lo, long long row_hi, float threshold,
-                    long long id_offset, long long cand_cap, long long* out_pairs, float* out_scores, long long out_cap,
-                    unsigned long long* out_count, int* out_overflowed, void* ws, size_t ws_bytes, int sm_count,
-                    cudaStream_t stream) {
+// Query rows [q_row_lo, q_row_hi) of `qdb` against the n_rows target rows of `db` (TRIANGLE when qdb == db and the id offsets
+// are equal, RECTANGLE otherwise: the caller guarantees disjoint row sets).  append == false: *out_count and *out_overflowed
+// are reset first (rvo_selfjoin_threshold[_ex]); append == true: pairs are appended at *out_count and overflowed candidate
+// sub-lists are added to *out_overflowed (rvo_join_threshold: every join of a device shares one pair buffer).
+int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi, long long q_id_offset, const uint16_t* db,
+                    long long n_rows, int d, float threshold, long long id_offset, long long cand_cap, long long* out_pairs,
+                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, bool append,
+                    void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream) {
     SelfJoinPlan sp;
     int rc = selfjoin_plan(d, cand_cap, ws, ws_bytes, &sp);
     if (rc) return rc;
-    RVO_CUDA(cudaMemsetAsync(out_count, 0, sizeof(unsigned long long), stream));
-    RVO_CUDA(cudaMemsetAsync(sp.overflowed, 0, sizeof(int), stream));
+    const bool triangle = qdb == db && q_id_offset == id_offset;
+    int* overflowed = append ? out_overflowed : sp.overflowed;
+    if (!append) {
+        RVO_CUDA(cudaMemsetAsync(out_count, 0, sizeof(unsigned long long), stream));
+        RVO_CUDA(cudaMemsetAsync(sp.overflowed, 0, sizeof(int), stream));
+    }
     const int nk = sp.d_pad / kTileCols;
-    for (long long i0 = row_lo; i0 < row_hi; i0 += kSelfJoinBlock) {
-        const int nq = (int)((row_hi - i0) < kSelfJoinBlock ? (row_hi - i0) : kSelfJoinBlock);
-        gather_rows_kernel<<<sp.tc.nq_pad, 256, 0, stream>>>((const uint4*)db, i0, nq, sp.tc.nq_pad, sp.d_pad, (uint4*)sp.qb,
+    for (long long i0 = q_row_lo; i0 < q_row_hi; i0 += kSelfJoinBlock) {
+        const int nq = (int)((q_row_hi - i0) < kSelfJoinBlock ? (q_row_hi - i0) : kSelfJoinBlock);
+        gather_rows_kernel<<<sp.tc.nq_pad, 256, 0, stream>>>((const uint4*)qdb, i0, nq, sp.tc.nq_pad, sp.d_pad, (uint4*)sp.qb,
                                                              sp.tau, threshold - kSelfJoinMargin);
         RVO_LAUNCHED();
         RVO_CUDA(cudaMemsetAsync(sp.cnt, 0, (size_t)sp.tc.nq_pad * kCandSplit * sizeof(int), stream));
-        // upper triangle: scan only the 128-row blocks at or after the first query row of this block
-        const long long blk0 = i0 / kTileRows;
+        // upper triangle: scan only the 128-row blocks at or after the first query row of this block; rectangle: every row
+        const long long blk0 = triangle ? i0 / kTileRows : 0;
         const long long scan_base = blk0 * kTileRows;
         const uint16_t* db_sub = db + (size_t)blk0 * nk * kTileRows * kTileCols;
         rc = launch_scan_tc(kModeFilter, db_sub, n_rows - scan_base, 1, sp.d_pad, sp.qb, sp.tc, sp.tau, sp.cand, sp.cnt, sp.cap,
                             nullptr, 0, sm_count, stream);
         if (rc) return rc;
         pairs_kernel<<<nq, 256, 0, stream>>>((const uint4*)db, (const uint4*)sp.qb, i0, scan_base, sp.d_pad, sp.cand, sp.cnt,
-                                             sp.cap, threshold, id_offset, out_pairs, out_scores, out_cap, out_count,
-                                             sp.overflowed);
+                                             sp.cap, threshold, triangle, q_id_offset, id_offset, out_pairs, out_scores, out_cap,
+                                             out_count, overflowed);
         RVO_LAUNCHED();
     }
-    if (out_overflowed)
+    if (!append && out_overflowed)
         RVO_CUDA(cudaMemcpyAsync(out_overflowed, sp.overflowed, sizeof(int), cudaMemcpyDeviceToDevice, stream));
     return RVO_OK;
 }

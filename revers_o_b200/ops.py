@@ -359,6 +359,34 @@ def selfjoin_exact(db: torch.Tensor, n_rows: int, d: int, threshold: float, row_
         return pairs[:m].cpu().numpy(), scores[:m].cpu().numpy()
 
 
+def join_out(out_cap: int, device) -> tuple:
+    """Pair buffer of `join_threshold`: (pairs int64 [out_cap, 2], scores f32 [out_cap], count int64 [1] = 0,
+    overflowed int32 [1] = 0)."""
+    return (torch.empty((out_cap, 2), dtype=torch.int64, device=device), torch.empty((out_cap,), dtype=torch.float32, device=device),
+            torch.zeros((1,), dtype=torch.int64, device=device), torch.zeros((1,), dtype=torch.int32, device=device))
+
+
+def join_threshold(qdb: torch.Tensor, q_row_lo: int, q_row_hi: int, q_id_offset: int, db: torch.Tensor, n_rows: int, d: int,
+                   threshold: float, id_offset: int, cand_cap: int, out: tuple) -> None:
+    """rvo_join_threshold: query rows [q_row_lo, q_row_hi) of the tiled storage `qdb` against the first n_rows rows of the tiled
+    storage `db`, pairs with cos >= threshold as (lower id, higher id), ids = row + offset.  `qdb is db` with equal offsets is the
+    triangle of the self-join (i < j only); otherwise the two row sets must be disjoint and every pair counts.  `out` (`join_out`,
+    on db's device) is APPENDED to: its count and overflow counter are never reset.  Async on the current stream of db's device."""
+    require_cuda(db, "db")
+    require_cuda(qdb, "qdb")
+    for t in (qdb, db):
+        assert t.dtype == torch.bfloat16 and t.dim() == 4 and t.is_contiguous() and t.shape[1] * TILE_COLS == d_pad_of(d)
+    assert n_rows <= db_capacity(db) and q_row_hi <= db_capacity(qdb)
+    pairs, scores, count, over = out
+    dev = db.device
+    lib = _lib.load()
+    nbytes = lib.rvo_join_workspace_bytes(d, int(cand_cap))
+    ws = workspace(dev, nbytes)
+    check(lib.rvo_join_threshold(_ptr(qdb), int(q_row_lo), int(q_row_hi), int(q_id_offset), _ptr(db), int(n_rows), d, d_pad_of(d),
+                                 float(threshold), int(id_offset), int(cand_cap), _ptr(pairs), _ptr(scores), pairs.shape[0],
+                                 _ptr(count), _ptr(over), _ptr(ws), nbytes, _stream(dev)), "rvo_join_threshold")
+
+
 def merge_topk(ids: torch.Tensor, scores: torch.Tensor, counts: torch.Tensor, k: int):
     """K3.  ids int64 [G,nq,k], scores f32 [G,nq,k], counts int32 [G,nq] -> merged (ids, scores, counts)."""
     require_cuda(ids, "ids")

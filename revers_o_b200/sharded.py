@@ -8,11 +8,17 @@ computes the same answer).  No other collective is on the data path.
 `shard_bounds`, `pack_results`, `unpack_results` and `allgather_packed` are backend-agnostic host
 logic (exercised with gloo on CPU in tests/test_sharded_gloo.py); `ShardedIndex.search` is the CUDA
 product path.
+
+The self-join of a collection row-sharded over the devices of ONE process (B200VectorDB(devices=[...]).find_near_duplicates) is
+here too: `selfjoin_plan` (pure host logic) and `selfjoin_sharded`, which joins the shards where they live and moves only
+query blocks.
 """
 from __future__ import annotations
 
 import ctypes as C
+from typing import NamedTuple
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -76,6 +82,198 @@ def selfjoin_blocks(n_rows: int, world: int, rank: int, block: int = 4096) -> li
         else:
             out.append((lo, hi))
     return out
+
+
+class JoinItem(NamedTuple):
+    """Query rows [q_lo, q_hi) of shard q_shard against target rows [t_lo, t_hi) of shard t_shard (local rows); it runs on the
+    target shard's device.  q_shard == t_shard: a block of that shard's triangle (pairs i < j only, t_lo = q_lo, t_hi = the
+    shard's size); otherwise a rectangle (every pair)."""
+    q_shard: int
+    q_lo: int
+    q_hi: int
+    t_shard: int
+    t_lo: int
+    t_hi: int
+
+
+def selfjoin_plan(sizes: list[int], block: int = 4096) -> list[list[JoinItem]]:
+    """Work of the self-join of a collection row-sharded into shards of `sizes` rows: list g holds the items that run on shard
+    g's device.  Every unordered pair of rows is examined by exactly one item, and no shard leaves its device: only query
+    blocks of `block` rows (a multiple of 128) move.
+
+    The triangle of a shard runs on its own device.  The rectangle of shards a < b is split at s, a multiple of `block`: query
+    blocks [0, s) of a run on b against all of b, and every query block of b runs on a against rows [s, n_a) of a (a target
+    sub-range that starts on a 128-row block).  s is chosen so that the devices' loads, in row pairs, are as even as the
+    triangles allow: the fractional shares are balanced pairwise until they settle (each step equalises the loads of the two
+    devices of one rectangle, which minimises the sum of squared loads and with it the largest), then rounded to whole
+    blocks one rectangle at a time."""
+    G = len(sizes)
+    n = [int(x) for x in sizes]
+    load = [x * (x - 1) / 2 for x in n]
+    rects = [(a, b) for a in range(G) for b in range(a + 1, G) if n[a] and n[b]]
+    share = {}                                   # share of rectangle (a, b) that runs on b
+    for a, b in rects:
+        share[a, b] = 0.5
+        load[a] += n[a] * n[b] / 2
+        load[b] += n[a] * n[b] / 2
+    for _ in range(200):
+        moved = 0.0
+        for a, b in rects:
+            r, x = n[a] * n[b], share[a, b]
+            la, lb = load[a] - (1 - x) * r, load[b] - x * r
+            v = min(1.0, max(0.0, (la - lb + r) / (2 * r)))
+            share[a, b] = v
+            load[a], load[b] = la + (1 - v) * r, lb + v * r
+            moved = max(moved, abs(v - x) * r)
+        if moved < 1.0:
+            break
+    split = {}
+    for a, b in rects:
+        r, x = n[a] * n[b], share[a, b]
+        la, lb = load[a] - (1 - x) * r, load[b] - x * r
+        lo = int(x * n[a]) // block * block
+        s = min((min(c, n[a]) for c in (lo, lo + block)), key=lambda c: (max(la + (n[a] - c) * n[b], lb + c * n[b]), c))
+        split[a, b] = s
+        load[a], load[b] = la + (n[a] - s) * n[b], lb + s * n[b]
+    plan: list[list[JoinItem]] = [[] for _ in range(G)]
+    for g in range(G):
+        plan[g] += [JoinItem(g, lo, min(lo + block, n[g]), g, lo, n[g]) for lo in range(0, n[g], block)]
+    for a, b in rects:
+        s = split[a, b]
+        plan[b] += [JoinItem(a, lo, min(lo + block, s), b, 0, n[b]) for lo in range(0, s, block)]
+        if s < n[a]:
+            plan[a] += [JoinItem(b, lo, min(lo + block, n[b]), a, s, n[a]) for lo in range(0, n[b], block)]
+    return plan
+
+
+def selfjoin_sharded(shards: list, d: int, threshold: float, max_pairs: int = 1 << 22, cand_cap: int = 32768,
+                     block: int = 4096, device_ms: dict | None = None):
+    """Self-join of a collection row-sharded over the devices of one process: all pairs of rows with cos >= threshold.
+    shards: [(tiled storage, rows, first global row)], each tensor on its shard's device (several shards may share a device).
+    Returns host arrays (pairs int64 [m, 2] of global rows, lower first; scores f32 [m]) — the same pairs and bit-identical
+    scores as the single-device join of the same rows.
+
+    Every item of `selfjoin_plan` is enqueued, round-robin over the devices, before any synchronisation: one host sync per
+    device.  A query block of another device is copied (a peer copy) into one of two staging blocks on the target device,
+    ordered after the source device's current stream; the joins run on each device's current stream and append to one pair
+    buffer per device.  Overflow protocol of `ops.selfjoin_exact`, judged per device: overflowed candidate lists re-run that
+    device's items with 8x the capacity (exact once it covers the rows scanned + 4096), a pair count above the buffer re-runs
+    them with a buffer of that count.  `device_ms`: filled with each device's busy time (CUDA events, ms) of the last attempt."""
+    sizes = [int(n) for _, n, _ in shards]
+    plan = selfjoin_plan(sizes, block)
+    items: dict[int, list[JoinItem]] = {}
+    for g, its in enumerate(plan):
+        items.setdefault(shards[g][0].device.index, []).extend(its)
+    cap = {dv: int(cand_cap) for dv in items}
+    out_cap = {dv: int(max_pairs) for dv in items}
+    rows_scanned = {dv: max(it.t_hi - it.t_lo for it in its) for dv, its in items.items() if its}
+    todo = sorted(rows_scanned)
+    done: dict[int, tuple] = {}
+    while todo:
+        ready = {}           # copies read a shard after what its device's current stream had queued before the join
+        for v, _, _ in shards:
+            if v.device.index not in ready:
+                ready[v.device.index] = torch.cuda.Event()
+                ready[v.device.index].record(torch.cuda.current_stream(v.device))
+        runs = {dv: _join_runs(items[dv], shards, dv) for dv in todo}
+        st = {dv: _JoinState(torch.device("cuda", dv), out_cap[dv], d, block, ready) for dv in todo}
+        for k in range(max(len(r) for r in runs.values())):
+            for dv in todo:
+                if k < len(runs[dv]):
+                    st[dv].run(runs[dv][k], shards, d, threshold, cap[dv])
+        retry = []
+        for dv in todo:
+            s = st[dv]
+            s.stop.record(torch.cuda.current_stream(s.dev))
+            torch.cuda.current_stream(s.dev).synchronize()
+            if device_ms is not None:
+                device_ms[dv] = s.start.elapsed_time(s.stop)
+            pairs, scores, count, over = s.out
+            m, ov = int(count.item()), int(over.item())
+            if ov > 0 and cap[dv] < rows_scanned[dv] + 4096:
+                cap[dv] = min(cap[dv] * 8, rows_scanned[dv] + 4096 + ops.TILE_ROWS * 16)
+                retry.append(dv)
+            elif m > out_cap[dv]:
+                out_cap[dv] = m
+                retry.append(dv)
+            elif ov > 0:
+                raise _lib.RvoError(f"self-join candidate lists overflowed at capacity {cap[dv]} on cuda:{dv}")
+            else:
+                done[dv] = (pairs[:m].cpu().numpy(), scores[:m].cpu().numpy())
+        todo = retry
+    if not done:
+        return np.zeros((0, 2), np.int64), np.zeros(0, np.float32)
+    return np.concatenate([done[dv][0] for dv in sorted(done)]), np.concatenate([done[dv][1] for dv in sorted(done)])
+
+
+def _join_runs(its: list[JoinItem], shards: list, dv: int) -> list[JoinItem]:
+    """The items of one device as calls: consecutive items that read their query rows in place (same device) and share a
+    target merge into one call (the C entry walks the query blocks itself); a query block of another device stays one call."""
+    runs: list[JoinItem] = []
+    for it in its:
+        local = shards[it.q_shard][0].device.index == dv
+        p = runs[-1] if runs else None
+        if (local and p is not None and shards[p.q_shard][0].device.index == dv and p.q_shard == it.q_shard
+                and p.t_shard == it.t_shard and p.q_hi == it.q_lo and p.t_hi == it.t_hi
+                and (p.t_lo == it.t_lo or it.q_shard == it.t_shard)):
+            runs[-1] = p._replace(q_hi=it.q_hi)
+        else:
+            runs.append(it)
+    return runs
+
+
+class _JoinState:
+    """Pair buffer, staging blocks and streams of one device during `selfjoin_sharded`."""
+
+    def __init__(self, dev: torch.device, out_cap: int, d: int, block: int, ready: dict):
+        self.dev, self.ready = dev, ready
+        self.out = ops.join_out(out_cap, dev)
+        self.d, self.block = d, block
+        self.slots: list = []                    # two staging blocks: the copy of one overlaps the join of the other
+        self.free: list = []                     # event per slot: the join that last read it has finished
+        self.next = 0
+        self.copy_stream = None
+        self.src_streams: dict = {}
+        self.start, self.stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        self.start.record(torch.cuda.current_stream(dev))
+
+    def run(self, it: JoinItem, shards: list, d: int, threshold: float, cand_cap: int) -> None:
+        qv, _, q_row0 = shards[it.q_shard]
+        tv, _, t_row0 = shards[it.t_shard]
+        cur = torch.cuda.current_stream(self.dev)
+        if it.q_shard == it.t_shard:
+            with torch.cuda.device(self.dev):
+                ops.join_threshold(tv, it.q_lo, it.q_hi, t_row0, tv, it.t_hi, d, threshold, t_row0, cand_cap, self.out)
+            return
+        target = tv[it.t_lo // ops.TILE_ROWS:]
+        if qv.device == self.dev:
+            qdb, q_lo, q_hi, q_off = qv, it.q_lo, it.q_hi, q_row0
+        else:
+            b0, b1 = it.q_lo // ops.TILE_ROWS, (it.q_hi + ops.TILE_ROWS - 1) // ops.TILE_ROWS
+            if not self.slots:
+                self.slots = [ops.db_alloc(self.block, d, self.dev) for _ in range(2)]
+                self.free = [None, None]
+                self.copy_stream = torch.cuda.Stream(self.dev)
+            k = self.next % 2
+            self.next += 1
+            src = self.src_streams.get(qv.device.index)
+            if src is None:
+                src = self.src_streams[qv.device.index] = torch.cuda.Stream(qv.device)
+                src.wait_event(self.ready[qv.device.index])
+            if self.free[k] is not None:
+                self.copy_stream.wait_event(self.free[k])
+            # a cross-device copy_ runs on the source device's current stream, after the destination device's current stream
+            with torch.cuda.stream(src), torch.cuda.stream(self.copy_stream):
+                self.slots[k][: b1 - b0].copy_(qv[b0:b1], non_blocking=True)
+            cur.wait_stream(self.copy_stream)
+            qdb, q_lo, q_hi, q_off = self.slots[k], it.q_lo - b0 * ops.TILE_ROWS, it.q_hi - b0 * ops.TILE_ROWS, q_row0 + b0 * ops.TILE_ROWS
+        with torch.cuda.device(self.dev):
+            ops.join_threshold(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo, cand_cap,
+                               self.out)
+        if qdb is not qv:
+            ev = torch.cuda.Event()
+            ev.record(cur)
+            self.free[k] = ev
 
 
 class ShardedIndex:

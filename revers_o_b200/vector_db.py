@@ -689,12 +689,16 @@ class B200VectorDB:
         """All pairs of stored points with cosine >= threshold (BASELINE config 4: keyframe near-duplicate self-join;
         generalises `score_threshold`, core_system.py:663).  Returns (list of (id_a, id_b), scores float32 [n]).  A row with more
         near-duplicates than the candidate lists hold (a static scene: thousands of identical frames) is re-joined exactly with
-        a larger list instead of failing."""
+        a larger list instead of failing.  A row-sharded collection is joined where it lives (`sharded.selfjoin_sharded`: each
+        shard with itself on its device, every pair of shards split between their two devices, only 4096-row query blocks
+        copied), with the same pairs and scores as on one device."""
         with self._lock.read():
             c = self._coll(collection_name)
-            if sum(1 for s in c.shards if s.n) > 1:
-                raise RvoError("find_near_duplicates needs the collection on one device (the join replicates the DB): load it with a "
-                               "single device")
+            active = [s for s in c.shards if s.n]
+            if len(active) > 1:
+                from .sharded import selfjoin_sharded
+                p, sc = selfjoin_sharded([(s.vectors, s.n, s.row0) for s in active], c.dim, threshold, max_pairs=max_pairs)
+                return [(c.ids[int(a)], c.ids[int(b)]) for a, b in p], sc
             s = next((s for s in c.shards if s.n), c.shards[0])
             n, vectors = s.n, s.vectors
             if n < 2:
