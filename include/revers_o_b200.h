@@ -300,6 +300,22 @@ int rvo_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, 
                        int64_t cand_cap, int64_t* out_pairs, float* out_scores, int64_t out_cap,
                        uint64_t* out_count, int32_t* out_overflowed, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Threshold join between two collections (left and right) on one device: every (query row, target row) pair with cos >= threshold.
+ *   qdb        [dev] tiled bf16 storage holding the query rows [q_row_lo, q_row_hi); their ids are row + q_id_offset
+ *   db         [dev] tiled bf16 storage of the n_rows target rows (a sub-range must start on a 128-row block); ids row + id_offset
+ *   query_is_right  0: the query rows are the left collection, 1: they are the right one
+ * A pair is stored as (left id, right id) whichever side provides the query rows, with the fp32 dot of its two stored bf16 rows;
+ * the score is bit-identical in both orientations (and equal to the self-join's score of the same two rows).  The ids of the two
+ * sides name rows of different collections, so they may overlap; qdb == db is allowed and is then the full ordered join of those
+ * rows with themselves, self pairs (i, i) included.  Both buffers must be on the same device.  Appends exactly like
+ * rvo_join_threshold (out_count and out_overflowed are added to, never reset); cand_cap and workspace
+ * (rvo_join_workspace_bytes(d, cand_cap) bytes, 1024-B aligned) as there. */
+int rvo_cross_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset,
+                             const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad, float threshold,
+                             int64_t id_offset, int32_t query_is_right, int64_t cand_cap,
+                             int64_t* out_pairs, float* out_scores, int64_t out_cap, uint64_t* out_count,
+                             int32_t* out_overflowed, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Counters for bench.py's `gpu_launches` claim: number of kernels THIS library has launched on the
  * calling process since load (monotonic).

@@ -573,6 +573,54 @@ class SimpleReverso:
             out.append(hits)
         return f"🎯 Searched {len(q)} regions", out
 
+    def find_shared_regions(self, other_database_name, similarity_threshold=0.95, max_results=20):
+        """New: which regions of the loaded database also appear in another database — every pair at cosine >=
+        similarity_threshold, found by one join on the GPU (`B200VectorDB.join_collections`) instead of one search per stored
+        region.  The other database is opened as `load_database` opens one (same devices, same collection naming).  Returns
+        (status text, list of dict{score, filename, bbox, other_filename, other_bbox}) for the `max_results` best pairs: score
+        descending, ties by the loaded database's row, then the other database's row."""
+        if not self.vector_db or not self.current_database:
+            return "❌ No database loaded. Please create or load a database first.", []
+        if not other_database_name:
+            return "❌ Please provide a database name", []
+        db_path = f"{self.db_root}/{other_database_name}"
+        if not os.path.exists(db_path):
+            return f"❌ Database not found: {other_database_name}", []
+        if self.vector_db.path and os.path.realpath(self.vector_db.path) == os.path.realpath(db_path):
+            return f"❌ {other_database_name} is the loaded database: choose another database to compare with", []
+        other = None
+        try:
+            other = self._new_client(db_path)
+            collection_name = f"{COLLECTION_PREFIX}{other_database_name}"
+            names = [c.name for c in other.get_collections().collections]
+            if collection_name not in names:
+                if other_database_name in names:  # legacy naming, as in load_database
+                    collection_name = other_database_name
+                else:
+                    return f"❌ Collection not found in database: {other_database_name}", []
+            print(f"🔍 Joining {self.current_database} with {collection_name} (threshold={similarity_threshold})")
+            with self.vector_db._read_both(other):
+                a, b, pairs, scores = self.vector_db._join_rows(self.current_database, collection_name, similarity_threshold,
+                                                               1 << 22, other)
+                best = np.lexsort((pairs[:, 1], pairs[:, 0], -scores))[:max(int(max_results), 0)]
+                items = []
+                for k in best:
+                    pa, pb = a.payloads[int(pairs[k, 0])] or {}, b.payloads[int(pairs[k, 1])] or {}
+                    items.append({"score": float(scores[k]), "filename": pa.get("filename", "Unknown"), "bbox": pa.get("bbox"),
+                                  "other_filename": pb.get("filename", "Unknown"), "other_bbox": pb.get("bbox")})
+        except Exception as e:
+            return f"❌ Join error: {e}", []
+        finally:
+            if other is not None:
+                other.close()
+        if len(pairs) == 0:
+            return f"❌ No shared regions found above threshold {similarity_threshold}", []
+        results_text = f"🎯 Found {len(pairs)} shared regions with {other_database_name}, showing {len(items)}:\n\n"
+        for i, it in enumerate(items):
+            results_text += f"{i + 1}. {it['filename']} ↔ {it['other_filename']} (Similarity: {it['score']:.3f})\n"
+            results_text += f"   📍 Bounding boxes: {it['bbox']} ↔ {it['other_bbox']}\n\n"
+        return results_text, items
+
     def visualize_detections(self, image, selected_region_index=None):
         """core_system.py:719-757 — rendering, out of scope; returns the image with region boxes drawn."""
         pil = self._to_pil(image).copy()

@@ -19,8 +19,8 @@ static std::atomic<long long> opt_select_trace{0};
 size_t selfjoin_workspace_bytes(int d, long long cand_cap);
 int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi, long long q_id_offset, const uint16_t* db,
                     long long n_rows, int d, float threshold, long long id_offset, long long cand_cap, long long* out_pairs,
-                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, bool append,
-                    void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream);
+                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, int mode,
+                    bool append, void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream);
 static thread_local char g_err[512] = "";
 std::atomic<long long> g_launches{0};
 std::atomic<long long> g_chain_trace{0};
@@ -860,8 +860,8 @@ int rvo_selfjoin_threshold_ex(const uint16_t* db, int64_t n_rows, int32_t d, int
     int rc = select_device_of(db, &sm);
     if (rc) return rc;
     return launch_selfjoin(db, row_lo, row_hi, id_offset, db, n_rows, d, threshold, id_offset, cand_cap, (long long*)out_pairs,
-                           out_scores, out_cap, (unsigned long long*)out_count, out_overflowed, false, workspace, workspace_bytes,
-                           sm, (cudaStream_t)stream);
+                           out_scores, out_cap, (unsigned long long*)out_count, out_overflowed, kJoinTriangle, false, workspace,
+                           workspace_bytes, sm, (cudaStream_t)stream);
 }
 
 size_t rvo_join_workspace_bytes(int32_t d, int64_t cand_cap) { return rvo_selfjoin_workspace_bytes_ex(d, cand_cap); }
@@ -908,8 +908,44 @@ int rvo_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, 
     int rc = select_device_of(db, &sm);
     if (rc) return rc;
     return launch_selfjoin(qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, threshold, id_offset, cand_cap,
-                           (long long*)out_pairs, out_scores, out_cap, (unsigned long long*)out_count, out_overflowed, true,
-                           workspace, workspace_bytes, sm, (cudaStream_t)stream);
+                           (long long*)out_pairs, out_scores, out_cap, (unsigned long long*)out_count, out_overflowed,
+                           triangle ? kJoinTriangle : kJoinRectangle, true, workspace, workspace_bytes, sm, (cudaStream_t)stream);
+}
+
+int rvo_cross_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset, const uint16_t* db,
+                             int64_t n_rows, int32_t d, int64_t d_pad_in, float threshold, int64_t id_offset,
+                             int32_t query_is_right, int64_t cand_cap, int64_t* out_pairs, float* out_scores, int64_t out_cap,
+                             uint64_t* out_count, int32_t* out_overflowed, void* workspace, size_t workspace_bytes,
+                             void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(qdb && db && out_pairs && out_scores && out_count && out_overflowed && workspace, "cross join: null pointer");
+    RVO_REQUIRE(n_rows > 0 && n_rows < (1ll << 31) && d > 0 && q_row_lo >= 0 && q_row_lo <= q_row_hi && out_cap >= 0 &&
+                    cand_cap > 0,
+                "cross join: bad shape n_rows=%lld query rows [%lld,%lld)", (long long)n_rows, (long long)q_row_lo,
+                (long long)q_row_hi);
+    RVO_REQUIRE(query_is_right == 0 || query_is_right == 1, "cross join: query_is_right must be 0 or 1, got %d",
+                (int)query_is_right);
+    RVO_REQUIRE(d_pad_in == (d + kBlockK - 1) / kBlockK * kBlockK, "cross join: d_pad must be d rounded up to 64");
+    RVO_REQUIRE(((uintptr_t)workspace & 1023) == 0 && ((uintptr_t)db & 15) == 0 && ((uintptr_t)qdb & 15) == 0,
+                "cross join: alignment");
+    // the two row sets belong to two collections: their ids may overlap, and qdb == db is the full ordered join of one row set
+    // with itself (self pairs included)
+    if (qdb == db)
+        RVO_REQUIRE(q_row_hi <= n_rows, "cross join: query rows [%lld,%lld) outside the %lld rows of the DB",
+                    (long long)q_row_lo, (long long)q_row_hi, (long long)n_rows);
+    int qdev = -1, tdev = -1;
+    int rc = select_device_of(qdb, nullptr);
+    if (rc) return rc;
+    RVO_CUDA(cudaGetDevice(&qdev));
+    int sm = 0;
+    rc = select_device_of(db, &sm);
+    if (rc) return rc;
+    RVO_CUDA(cudaGetDevice(&tdev));
+    RVO_REQUIRE(qdev == tdev, "cross join: query rows on device %d, target rows on device %d", qdev, tdev);
+    return launch_selfjoin(qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, threshold, id_offset, cand_cap,
+                           (long long*)out_pairs, out_scores, out_cap, (unsigned long long*)out_count, out_overflowed,
+                           query_is_right ? kJoinCrossRight : kJoinCrossLeft, true, workspace, workspace_bytes, sm,
+                           (cudaStream_t)stream);
 }
 
 int rvo_merge_topk(const int64_t* ids, const float* scores, const int32_t* counts, int32_t G, int32_t nq, int32_t k,

@@ -162,4 +162,9 @@ __host__ __device__ __forceinline__ float query_margin(float bf16_err_norm) {
 // worst case of query_margin (||bf16(q)-q|| <= 2^-8 ||q||): used where no per-query value exists
 constexpr float kBf16QueryMargin = 0.0082f;
 
+// Threshold join modes (selfjoin.cu): the self-join's upper triangle, a rectangle between two disjoint row sets of one
+// collection (pairs as (lower id, higher id)), and a join across two collections with the query rows from the left or the
+// right collection (pairs as (left id, right id)).
+enum JoinMode : int { kJoinTriangle = 0, kJoinRectangle = 1, kJoinCrossLeft = 2, kJoinCrossRight = 3 };
+
 }  // namespace rvo

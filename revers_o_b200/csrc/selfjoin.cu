@@ -4,13 +4,16 @@
 //   per block of up to 4096 query rows:  gather the rows out of the tiled query buffer (they ARE bf16, so the tensor-core
 //   scores are exact up to fp32 summation order) -> FILTER scan of the target rows with tau = threshold - 1e-4 ->
 //   `pairs_kernel`: fp32 re-score of every candidate, append (min id, max id, score).
-// Two modes share that code:
+// Three modes share that code:
 //   TRIANGLE  query rows and target rows are the same tiled DB: block b scans only rows >= its first row and keeps j > i,
 //             i.e. N^2 * D flops, not 2 N^2 D.
 //   RECTANGLE the query rows come from another tiled buffer on the same device (a block of another shard copied here) and
 //             are disjoint from the target rows: every target row is scanned, every candidate re-scored.  Used for the
-//             cross-shard part of the join of a row-sharded collection.
-// The re-score runs the same lanes over the same chunks in the same order in both modes and fmaf is commutative in its two
+//             cross-shard part of the join of a row-sharded collection.  Pairs are stored as (lower id, higher id).
+//   CROSS     the query rows and the target rows belong to two different collections (left and right), so their ids may
+//             overlap and the buffers may even coincide: every target row is scanned, every candidate re-scored, and the pair
+//             is stored as (left id, right id) whichever side provides the query rows.
+// The re-score runs the same lanes over the same chunks in the same order in every mode and fmaf is commutative in its two
 // factors, so a pair scores bit-identically whichever of its rows is the query.
 #include "common.cuh"
 #include "scan_tc.cuh"
@@ -47,17 +50,18 @@ __device__ __forceinline__ float dot8(const uint4 a, const uint4 b, float acc) {
 }
 
 // grid (nq), 256 threads: candidates of query row i = row0 + q; 8 lanes per candidate.  j_floor: a candidate j is re-scored
-// when j > j_floor — the query row i in TRIANGLE mode (upper triangle, no self pair), -1 in RECTANGLE mode (every candidate).
-// Pairs are emitted as (min, max) of (i + q_id_offset, j + id_offset).
+// when j > j_floor — the query row i in TRIANGLE mode (upper triangle, no self pair), -1 otherwise (every candidate).
+// With gi = i + q_id_offset and gj = j + id_offset a pair is emitted as (min, max) of (gi, gj) in TRIANGLE and RECTANGLE mode,
+// as (gi, gj) in CROSS_LEFT (the query rows are the left collection) and as (gj, gi) in CROSS_RIGHT.
 __global__ void __launch_bounds__(256) pairs_kernel(const uint4* __restrict__ db, const uint4* __restrict__ qrows, long long row0,
                                                     long long scan_base, int d_pad, const unsigned long long* __restrict__ cand,
-                                                    const int* __restrict__ cnt, int cap, float threshold, bool triangle,
+                                                    const int* __restrict__ cnt, int cap, float threshold, int mode,
                                                     long long q_id_offset, long long id_offset, long long* __restrict__ out_pairs,
                                                     float* __restrict__ out_scores, long long out_cap,
                                                     unsigned long long* __restrict__ out_count, int* __restrict__ overflowed) {
     const int q = blockIdx.x;
     const long long i = row0 + q;
-    const long long j_floor = triangle ? i : -1;
+    const long long j_floor = mode == kJoinTriangle ? i : -1;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
     const int g = lane >> 3, l8 = lane & 7;
     const int nchunk = d_pad >> 3, nk = d_pad / kTileCols;
@@ -92,8 +96,9 @@ __global__ void __launch_bounds__(256) pairs_kernel(const uint4* __restrict__ db
                     const unsigned long long at = base + __popc(bal & ((1u << lane) - 1u));
                     if ((long long)at < out_cap) {
                         const long long gi = i + q_id_offset, gj = j + id_offset;
-                        out_pairs[2 * at] = gi < gj ? gi : gj;
-                        out_pairs[2 * at + 1] = gi < gj ? gj : gi;
+                        const bool swap = mode == kJoinCrossRight || (mode < kJoinCrossLeft && gj < gi);
+                        out_pairs[2 * at] = swap ? gj : gi;
+                        out_pairs[2 * at + 1] = swap ? gi : gj;
                         out_scores[at] = acc;
                     }
                 }
@@ -142,18 +147,18 @@ size_t selfjoin_workspace_bytes(int d, long long cand_cap) {
     return sp.bytes;
 }
 
-// Query rows [q_row_lo, q_row_hi) of `qdb` against the n_rows target rows of `db` (TRIANGLE when qdb == db and the id offsets
-// are equal, RECTANGLE otherwise: the caller guarantees disjoint row sets).  append == false: *out_count and *out_overflowed
-// are reset first (rvo_selfjoin_threshold[_ex]); append == true: pairs are appended at *out_count and overflowed candidate
+// Query rows [q_row_lo, q_row_hi) of `qdb` against the n_rows target rows of `db` in `mode` (JoinMode; the caller has checked
+// what the mode needs: TRIANGLE qdb == db with equal id offsets, RECTANGLE disjoint row sets).  append == false: *out_count and
+// *out_overflowed are reset first (rvo_selfjoin_threshold[_ex]); append == true: pairs are appended at *out_count and overflowed candidate
 // sub-lists are added to *out_overflowed (rvo_join_threshold: every join of a device shares one pair buffer).
 int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi, long long q_id_offset, const uint16_t* db,
                     long long n_rows, int d, float threshold, long long id_offset, long long cand_cap, long long* out_pairs,
-                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, bool append,
-                    void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream) {
+                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, int mode,
+                    bool append, void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream) {
     SelfJoinPlan sp;
     int rc = selfjoin_plan(d, cand_cap, ws, ws_bytes, &sp);
     if (rc) return rc;
-    const bool triangle = qdb == db && q_id_offset == id_offset;
+    const bool triangle = mode == kJoinTriangle;
     int* overflowed = append ? out_overflowed : sp.overflowed;
     if (!append) {
         RVO_CUDA(cudaMemsetAsync(out_count, 0, sizeof(unsigned long long), stream));
@@ -166,7 +171,7 @@ int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi,
                                                              sp.tau, threshold - kSelfJoinMargin);
         RVO_LAUNCHED();
         RVO_CUDA(cudaMemsetAsync(sp.cnt, 0, (size_t)sp.tc.nq_pad * kCandSplit * sizeof(int), stream));
-        // upper triangle: scan only the 128-row blocks at or after the first query row of this block; rectangle: every row
+        // upper triangle: scan only the 128-row blocks at or after the first query row of this block; otherwise every row
         const long long blk0 = triangle ? i0 / kTileRows : 0;
         const long long scan_base = blk0 * kTileRows;
         const uint16_t* db_sub = db + (size_t)blk0 * nk * kTileRows * kTileCols;
@@ -174,7 +179,7 @@ int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi,
                             nullptr, 0, sm_count, stream);
         if (rc) return rc;
         pairs_kernel<<<nq, 256, 0, stream>>>((const uint4*)db, (const uint4*)sp.qb, i0, scan_base, sp.d_pad, sp.cand, sp.cnt,
-                                             sp.cap, threshold, triangle, q_id_offset, id_offset, out_pairs, out_scores, out_cap,
+                                             sp.cap, threshold, mode, q_id_offset, id_offset, out_pairs, out_scores, out_cap,
                                              out_count, overflowed);
         RVO_LAUNCHED();
     }

@@ -387,6 +387,29 @@ def join_threshold(qdb: torch.Tensor, q_row_lo: int, q_row_hi: int, q_id_offset:
                                  _ptr(count), _ptr(over), _ptr(ws), nbytes, _stream(dev)), "rvo_join_threshold")
 
 
+def cross_join_threshold(qdb: torch.Tensor, q_row_lo: int, q_row_hi: int, q_id_offset: int, db: torch.Tensor, n_rows: int, d: int,
+                         threshold: float, id_offset: int, query_is_right: bool, cand_cap: int, out: tuple) -> None:
+    """rvo_cross_join_threshold: query rows [q_row_lo, q_row_hi) of the tiled storage `qdb` against the first n_rows rows of the
+    tiled storage `db`, where the two belong to different collections: every pair with cos >= threshold, stored as (left id,
+    right id) with ids = row + offset; `query_is_right` says which collection the query rows are.  The ids may overlap and
+    `qdb is db` is allowed (the full ordered join, self pairs included).  `out` (`join_out`, on db's device) is APPENDED to, as in
+    `join_threshold`.  Async on the current stream of db's device."""
+    require_cuda(db, "db")
+    require_cuda(qdb, "qdb")
+    for t in (qdb, db):
+        assert t.dtype == torch.bfloat16 and t.dim() == 4 and t.is_contiguous() and t.shape[1] * TILE_COLS == d_pad_of(d)
+    assert n_rows <= db_capacity(db) and q_row_hi <= db_capacity(qdb)
+    pairs, scores, count, over = out
+    dev = db.device
+    lib = _lib.load()
+    nbytes = lib.rvo_join_workspace_bytes(d, int(cand_cap))
+    ws = workspace(dev, nbytes)
+    check(lib.rvo_cross_join_threshold(_ptr(qdb), int(q_row_lo), int(q_row_hi), int(q_id_offset), _ptr(db), int(n_rows), d,
+                                       d_pad_of(d), float(threshold), int(id_offset), int(bool(query_is_right)), int(cand_cap),
+                                       _ptr(pairs), _ptr(scores), pairs.shape[0], _ptr(count), _ptr(over), _ptr(ws), nbytes,
+                                       _stream(dev)), "rvo_cross_join_threshold")
+
+
 def merge_topk(ids: torch.Tensor, scores: torch.Tensor, counts: torch.Tensor, k: int):
     """K3.  ids int64 [G,nq,k], scores f32 [G,nq,k], counts int32 [G,nq] -> merged (ids, scores, counts)."""
     require_cuda(ids, "ids")

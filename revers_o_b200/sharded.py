@@ -11,7 +11,8 @@ product path.
 
 The self-join of a collection row-sharded over the devices of ONE process (B200VectorDB(devices=[...]).find_near_duplicates) is
 here too: `selfjoin_plan` (pure host logic) and `selfjoin_sharded`, which joins the shards where they live and moves only
-query blocks.
+query blocks.  So is the join between two such collections (B200VectorDB.join_collections): `crossjoin_plan` and
+`crossjoin_sharded`, run by the same device loop.
 """
 from __future__ import annotations
 
@@ -96,6 +97,40 @@ class JoinItem(NamedTuple):
     t_hi: int
 
 
+def _split_rectangles(load, rects: list, block: int) -> dict:
+    """Split points of rectangles whose two sides live on two different devices.  rects: [(key, u, v, n_a, n_b)]: query blocks
+    [0, s) of side a run on v against all of side b, every query block of b runs on u against rows [s, n_a) of a.  `load`
+    (indexable by u and v) holds the loads, in row pairs, that are already fixed, and is updated with the rectangles' shares.
+    The fractional shares are balanced pairwise until they settle (each step equalises the loads of the two devices of one
+    rectangle, which minimises the sum of squared loads and with it the largest), then rounded to multiples of `block` one
+    rectangle at a time.  Returns {key: s}."""
+    share = {}                                   # share of each rectangle that runs on v
+    for key, u, v, na, nb in rects:
+        share[key] = 0.5
+        load[u] += na * nb / 2
+        load[v] += na * nb / 2
+    for _ in range(200):
+        moved = 0.0
+        for key, u, v, na, nb in rects:
+            r, x = na * nb, share[key]
+            lu, lv = load[u] - (1 - x) * r, load[v] - x * r
+            w = min(1.0, max(0.0, (lu - lv + r) / (2 * r)))
+            share[key] = w
+            load[u], load[v] = lu + (1 - w) * r, lv + w * r
+            moved = max(moved, abs(w - x) * r)
+        if moved < 1.0:
+            break
+    split = {}
+    for key, u, v, na, nb in rects:
+        r, x = na * nb, share[key]
+        lu, lv = load[u] - (1 - x) * r, load[v] - x * r
+        lo = int(x * na) // block * block
+        s = min((min(c, na) for c in (lo, lo + block)), key=lambda c: (max(lu + (na - c) * nb, lv + c * nb), c))
+        split[key] = s
+        load[u], load[v] = lu + (na - s) * nb, lv + s * nb
+    return split
+
+
 def selfjoin_plan(sizes: list[int], block: int = 4096) -> list[list[JoinItem]]:
     """Work of the self-join of a collection row-sharded into shards of `sizes` rows: list g holds the items that run on shard
     g's device.  Every unordered pair of rows is examined by exactly one item, and no shard leaves its device: only query
@@ -104,37 +139,12 @@ def selfjoin_plan(sizes: list[int], block: int = 4096) -> list[list[JoinItem]]:
     The triangle of a shard runs on its own device.  The rectangle of shards a < b is split at s, a multiple of `block`: query
     blocks [0, s) of a run on b against all of b, and every query block of b runs on a against rows [s, n_a) of a (a target
     sub-range that starts on a 128-row block).  s is chosen so that the devices' loads, in row pairs, are as even as the
-    triangles allow: the fractional shares are balanced pairwise until they settle (each step equalises the loads of the two
-    devices of one rectangle, which minimises the sum of squared loads and with it the largest), then rounded to whole
-    blocks one rectangle at a time."""
+    triangles allow (`_split_rectangles`, with one load per shard)."""
     G = len(sizes)
     n = [int(x) for x in sizes]
     load = [x * (x - 1) / 2 for x in n]
     rects = [(a, b) for a in range(G) for b in range(a + 1, G) if n[a] and n[b]]
-    share = {}                                   # share of rectangle (a, b) that runs on b
-    for a, b in rects:
-        share[a, b] = 0.5
-        load[a] += n[a] * n[b] / 2
-        load[b] += n[a] * n[b] / 2
-    for _ in range(200):
-        moved = 0.0
-        for a, b in rects:
-            r, x = n[a] * n[b], share[a, b]
-            la, lb = load[a] - (1 - x) * r, load[b] - x * r
-            v = min(1.0, max(0.0, (la - lb + r) / (2 * r)))
-            share[a, b] = v
-            load[a], load[b] = la + (1 - v) * r, lb + v * r
-            moved = max(moved, abs(v - x) * r)
-        if moved < 1.0:
-            break
-    split = {}
-    for a, b in rects:
-        r, x = n[a] * n[b], share[a, b]
-        la, lb = load[a] - (1 - x) * r, load[b] - x * r
-        lo = int(x * n[a]) // block * block
-        s = min((min(c, n[a]) for c in (lo, lo + block)), key=lambda c: (max(la + (n[a] - c) * n[b], lb + c * n[b]), c))
-        split[a, b] = s
-        load[a], load[b] = la + (n[a] - s) * n[b], lb + s * n[b]
+    split = _split_rectangles(load, [((a, b), a, b, n[a], n[b]) for a, b in rects], block)
     plan: list[list[JoinItem]] = [[] for _ in range(G)]
     for g in range(G):
         plan[g] += [JoinItem(g, lo, min(lo + block, n[g]), g, lo, n[g]) for lo in range(0, n[g], block)]
@@ -146,24 +156,80 @@ def selfjoin_plan(sizes: list[int], block: int = 4096) -> list[list[JoinItem]]:
     return plan
 
 
+def crossjoin_plan(left: list, right: list, block: int = 4096) -> dict[int, list[JoinItem]]:
+    """Work of the join between two row-sharded collections: left and right are [(device index, rows)], one entry per shard
+    (several shards may share a device, and the two sides may list different devices).  Returns {device index: items that
+    run there} for every device listed.  An item's shard index counts the left shards first: shard a of the left side is
+    a, shard b of the right side is len(left) + b.  Every (left row, right row) pair is examined by exactly one item, and
+    only query blocks of `block` rows (a multiple of 128) move.
+
+    The rectangle of left shard a and right shard b runs whole on their device when they share one (left query blocks
+    against all of b).  Otherwise it is split at s, a multiple of `block`: left query blocks [0, s) of a run on b's device
+    against all of b, and every query block of b runs on a's device against left rows [s, n_a) (a target sub-range that
+    starts on a 128-row block).  The loads are the devices' (`_split_rectangles`, one load per device)."""
+    L = [(int(dv), int(n)) for dv, n in left]
+    R = [(int(dv), int(n)) for dv, n in right]
+    nl = len(L)
+    plan: dict[int, list[JoinItem]] = {}
+    for dv, _ in L + R:
+        plan.setdefault(dv, [])
+    load = {dv: 0.0 for dv in plan}
+    rects = []
+    for a, (da, na) in enumerate(L):
+        for b, (db, nb) in enumerate(R):
+            if not na or not nb:
+                continue
+            if da == db:
+                load[da] += na * nb
+                plan[da] += [JoinItem(a, lo, min(lo + block, na), nl + b, 0, nb) for lo in range(0, na, block)]
+            else:
+                rects.append(((a, b), da, db, na, nb))
+    split = _split_rectangles(load, rects, block)
+    for (a, b), da, db, na, nb in rects:
+        s = split[a, b]
+        plan[db] += [JoinItem(a, lo, min(lo + block, s), nl + b, 0, nb) for lo in range(0, s, block)]
+        if s < na:
+            plan[da] += [JoinItem(nl + b, lo, min(lo + block, nb), a, s, na) for lo in range(0, nb, block)]
+    return plan
+
+
 def selfjoin_sharded(shards: list, d: int, threshold: float, max_pairs: int = 1 << 22, cand_cap: int = 32768,
                      block: int = 4096, device_ms: dict | None = None):
     """Self-join of a collection row-sharded over the devices of one process: all pairs of rows with cos >= threshold.
     shards: [(tiled storage, rows, first global row)], each tensor on its shard's device (several shards may share a device).
     Returns host arrays (pairs int64 [m, 2] of global rows, lower first; scores f32 [m]) — the same pairs and bit-identical
-    scores as the single-device join of the same rows.
-
-    Every item of `selfjoin_plan` is enqueued, round-robin over the devices, before any synchronisation: one host sync per
-    device.  A query block of another device is copied (a peer copy) into one of two staging blocks on the target device,
-    ordered after the source device's current stream; the joins run on each device's current stream and append to one pair
-    buffer per device.  Overflow protocol of `ops.selfjoin_exact`, judged per device: overflowed candidate lists re-run that
-    device's items with 8x the capacity (exact once it covers the rows scanned + 4096), a pair count above the buffer re-runs
-    them with a buffer of that count.  `device_ms`: filled with each device's busy time (CUDA events, ms) of the last attempt."""
+    scores as the single-device join of the same rows.  Runs the items of `selfjoin_plan` through `_join_on_devices`."""
     sizes = [int(n) for _, n, _ in shards]
     plan = selfjoin_plan(sizes, block)
     items: dict[int, list[JoinItem]] = {}
     for g, its in enumerate(plan):
         items.setdefault(shards[g][0].device.index, []).extend(its)
+    return _join_on_devices(shards, items, d, threshold, max_pairs, cand_cap, block, device_ms, None)
+
+
+def crossjoin_sharded(left: list, right: list, d: int, threshold: float, max_pairs: int = 1 << 22, cand_cap: int = 32768,
+                      block: int = 4096, device_ms: dict | None = None):
+    """Join of two collections, each row-sharded over devices of one process (one shard on one device is the plain case):
+    all (left row, right row) pairs with cos >= threshold.  left, right: [(tiled storage, rows, first global row)].  Returns
+    host arrays (pairs int64 [m, 2] = (left global row, right global row); scores f32 [m], the fp32 dot of the two stored
+    rows, bit-identical to the self-join's score of the same rows).  Runs the items of `crossjoin_plan` through
+    `_join_on_devices`."""
+    items = crossjoin_plan([(v.device.index, n) for v, n, _ in left], [(v.device.index, n) for v, n, _ in right], block)
+    return _join_on_devices(list(left) + list(right), items, d, threshold, max_pairs, cand_cap, block, device_ms, len(left))
+
+
+def _join_on_devices(shards: list, items: dict, d: int, threshold: float, max_pairs: int, cand_cap: int, block: int,
+                     device_ms: dict | None, n_left: int | None):
+    """Run {device index: [JoinItem]} over shards [(tiled storage, rows, first global row)].  n_left None: the items are a
+    self-join's (triangles and rectangles, `rvo_join_threshold`); otherwise shards [0, n_left) are the left collection and
+    the rest the right one, and every item is a cross join (`rvo_cross_join_threshold`).
+
+    Every item is enqueued, round-robin over the devices, before any synchronisation: one host sync per device.  A query
+    block of another device is copied (a peer copy) into one of two staging blocks on the target device, ordered after the
+    source device's current stream; the joins run on each device's current stream and append to one pair buffer per device.
+    Overflow protocol of `ops.selfjoin_exact`, judged per device: overflowed candidate lists re-run that device's items with
+    8x the capacity (exact once it covers the rows scanned + 4096), a pair count above the buffer re-runs them with a buffer
+    of that count.  `device_ms`: filled with each device's busy time (CUDA events, ms) of the last attempt."""
     cap = {dv: int(cand_cap) for dv in items}
     out_cap = {dv: int(max_pairs) for dv in items}
     rows_scanned = {dv: max(it.t_hi - it.t_lo for it in its) for dv, its in items.items() if its}
@@ -176,7 +242,7 @@ def selfjoin_sharded(shards: list, d: int, threshold: float, max_pairs: int = 1 
                 ready[v.device.index] = torch.cuda.Event()
                 ready[v.device.index].record(torch.cuda.current_stream(v.device))
         runs = {dv: _join_runs(items[dv], shards, dv) for dv in todo}
-        st = {dv: _JoinState(torch.device("cuda", dv), out_cap[dv], d, block, ready) for dv in todo}
+        st = {dv: _JoinState(torch.device("cuda", dv), out_cap[dv], d, block, ready, n_left) for dv in todo}
         for k in range(max(len(r) for r in runs.values())):
             for dv in todo:
                 if k < len(runs[dv]):
@@ -197,7 +263,8 @@ def selfjoin_sharded(shards: list, d: int, threshold: float, max_pairs: int = 1 
                 out_cap[dv] = m
                 retry.append(dv)
             elif ov > 0:
-                raise _lib.RvoError(f"self-join candidate lists overflowed at capacity {cap[dv]} on cuda:{dv}")
+                what = "self-join" if n_left is None else "cross join"
+                raise _lib.RvoError(f"{what} candidate lists overflowed at capacity {cap[dv]} on cuda:{dv}")
             else:
                 done[dv] = (pairs[:m].cpu().numpy(), scores[:m].cpu().numpy())
         todo = retry
@@ -223,10 +290,10 @@ def _join_runs(its: list[JoinItem], shards: list, dv: int) -> list[JoinItem]:
 
 
 class _JoinState:
-    """Pair buffer, staging blocks and streams of one device during `selfjoin_sharded`."""
+    """Pair buffer, staging blocks and streams of one device during `_join_on_devices`."""
 
-    def __init__(self, dev: torch.device, out_cap: int, d: int, block: int, ready: dict):
-        self.dev, self.ready = dev, ready
+    def __init__(self, dev: torch.device, out_cap: int, d: int, block: int, ready: dict, n_left: int | None = None):
+        self.dev, self.ready, self.n_left = dev, ready, n_left
         self.out = ops.join_out(out_cap, dev)
         self.d, self.block = d, block
         self.slots: list = []                    # two staging blocks: the copy of one overlaps the join of the other
@@ -268,8 +335,12 @@ class _JoinState:
             cur.wait_stream(self.copy_stream)
             qdb, q_lo, q_hi, q_off = self.slots[k], it.q_lo - b0 * ops.TILE_ROWS, it.q_hi - b0 * ops.TILE_ROWS, q_row0 + b0 * ops.TILE_ROWS
         with torch.cuda.device(self.dev):
-            ops.join_threshold(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo, cand_cap,
-                               self.out)
+            if self.n_left is None:
+                ops.join_threshold(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo, cand_cap,
+                                   self.out)
+            else:
+                ops.cross_join_threshold(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo,
+                                         it.q_shard >= self.n_left, cand_cap, self.out)
         if qdb is not qv:
             ev = torch.cuda.Event()
             ev.record(cur)

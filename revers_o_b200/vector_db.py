@@ -6,7 +6,9 @@ It duck-types exactly the five qdrant-client methods core_system.py uses (SURVEY
   .recreate_collection(collection_name, vectors_config=VectorParams(size, distance=COSINE))   :600-603
   .upsert(collection_name, points=[PointStruct(id, vector, payload)])                          :621
   .search(collection_name, query_vector, limit, score_threshold) -> [obj(.score,.payload)]     :659-664
-plus the batched entry point `search_batch` (new; reduces to `search` row by row, SURVEY.md F7).
+plus the batched entry point `search_batch` (new; reduces to `search` row by row, SURVEY.md F7), and two threshold joins
+(new): `find_near_duplicates` (every pair within one collection at cos >= threshold) and `join_collections` (every pair across
+two collections, possibly of two B200VectorDB instances: which regions of one archive also appear in another).
 
 Vectors live on the GPU(s) as L2-normalised bf16 rows in the TILED storage of include/revers_o_b200.h
 ([row/128][col/64][128][64]: one contiguous 16 KiB TMA box per tile; the DB is DEFINED as its bf16 values).  All arithmetic
@@ -33,7 +35,7 @@ import json
 import os
 import threading
 import weakref
-from contextlib import contextmanager
+from contextlib import ExitStack, contextmanager
 from dataclasses import dataclass
 from types import SimpleNamespace
 from typing import Any, Iterable
@@ -705,6 +707,45 @@ class B200VectorDB:
                 return [], np.zeros(0, np.float32)
             p, sc = ops.selfjoin_exact(vectors, n, c.dim, threshold, max_pairs=max_pairs, id_offset=s.row0)
             return [(c.ids[int(a)], c.ids[int(b)]) for a, b in p], sc
+
+    def join_collections(self, collection_name: str, other_collection_name: str, threshold: float = 0.95,
+                         max_pairs: int = 1 << 22, other: B200VectorDB | None = None):
+        """All pairs (point of `collection_name`, point of `other_collection_name`) with cosine >= threshold: "which regions of
+        archive A also appear in archive B" in one call.  `other` is the B200VectorDB holding the second collection (revers-o
+        opens one per database); by default this one.  Returns (list of (left id, right id), scores float32 [m]) in no
+        particular order; a score is the fp32 dot of the two stored bf16 rows.  The two collections are joined where they live,
+        each possibly row-sharded over several devices (`sharded.crossjoin_sharded`: only 4096-row query blocks are copied), with
+        the same pairs and scores on any layout.  Both databases stay read-locked for the call."""
+        other = self if other is None else other
+        with self._read_both(other):
+            a, b, p, sc = self._join_rows(collection_name, other_collection_name, threshold, max_pairs, other)
+            return [(a.ids[int(i)], b.ids[int(j)]) for i, j in p], sc
+
+    @contextmanager
+    def _read_both(self, other: B200VectorDB):
+        """Read locks of this DB and `other`, taken in one fixed order (by object id) whichever side calls; once if other is self."""
+        dbs = [self] if other is self else sorted((self, other), key=id)
+        with ExitStack() as stack:
+            for db in dbs:
+                stack.enter_context(db._lock.read())
+            yield
+
+    def _join_rows(self, collection_name: str, other_collection_name: str, threshold: float, max_pairs: int, other: B200VectorDB):
+        """`join_collections` in rows; the caller holds both read locks.  Returns (left collection, right collection, pairs int64
+        [m, 2] of (left row, right row), scores float32 [m])."""
+        if other is self and collection_name == other_collection_name:
+            raise RvoError(f"join_collections joins two different collections: the near-duplicates within {collection_name} "
+                           "are find_near_duplicates(collection_name)")
+        a, b = self._coll(collection_name), other._coll(other_collection_name)
+        if b.dim != a.dim:
+            raise RvoError(f"Wrong input: Vector dimension error: expected dim: {a.dim}, got {b.dim}")
+        left = [(s.vectors, s.n, s.row0) for s in a.shards if s.n]
+        right = [(s.vectors, s.n, s.row0) for s in b.shards if s.n]
+        if not left or not right:
+            return a, b, np.zeros((0, 2), np.int64), np.zeros(0, np.float32)
+        from .sharded import crossjoin_sharded
+        p, sc = crossjoin_sharded(left, right, a.dim, threshold, max_pairs=max_pairs)
+        return a, b, p, sc
 
     def count(self, collection_name: str) -> int:
         return self._coll(collection_name).n
