@@ -266,6 +266,7 @@ int rvo_search_topk_fused(const uint16_t* db, int64_t n_rows, int32_t d, int64_t
  * (2) DB row-sharded over the devices of one process (B200VectorDB(devices=[...])): rvo_join_threshold below joins each shard
  * with itself (triangle) and every pair of shards (rectangle, 4096-row query blocks copied to the other shard's device, each
  * rectangle split between its two devices); no shard is moved or replicated.
+ * Duplicate groups (the connected components of these pairs) without storing any pair: rvo_join_components below.
  * ---------------------------------------------------------------------------------------------- */
 size_t rvo_selfjoin_workspace_bytes(int32_t d);
 int rvo_selfjoin_threshold(const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad, int64_t row_lo, int64_t row_hi,
@@ -315,6 +316,29 @@ int rvo_cross_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_ro
                              int64_t id_offset, int32_t query_is_right, int64_t cand_cap,
                              int64_t* out_pairs, float* out_scores, int64_t out_cap, uint64_t* out_count,
                              int32_t* out_overflowed, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Connected components of the self-join's pairs (single-linkage groups at a threshold), with no pair stored.
+ * rvo_join_components takes the arguments of rvo_join_threshold and examines exactly the pairs it would emit (same scan, same
+ * fp32 re-score, same >= threshold test, triangle or rectangle derived the same way), but unions the two global rows of each
+ * into a union-find forest instead of storing the pair:
+ *   parent     [dev] int32 [n_labels], indexed by global row (ids = row + offset, every one < n_labels < 2^31); initialise it
+ *              to parent[x] = x once, then any number of joins (of one device) may union into it.  The forest keeps
+ *              parent[x] <= x: a hook sets the larger of two roots to the smaller, so a component's root is its smallest row.
+ *   hit_count  [dev] uint64 [1]  pairs at or above the threshold, ADDED to (never reset), like rvo_join_threshold's out_count
+ *   out_overflowed  [dev] int32 [1]  overflowed candidate sub-lists, added to; > 0: edges may be missing, re-run with a larger
+ *              cand_cap (re-applying an edge changes nothing, so the forest may be kept; reset hit_count first)
+ * cand_cap and workspace (rvo_join_workspace_bytes(d, cand_cap) bytes, 1024-B aligned) as in rvo_join_threshold; parent must be
+ * on the target rows' device.
+ * rvo_components_flatten: labels_out[x] = root of x (int32 [n]): the canonical label, the smallest row of x's component.
+ * rvo_components_merge: union(x, labels_src[x]) for every x with labels_src[x] != x (int32 [n], entries outside [0, n)
+ * ignored): folds the flattened forest of another device over the same n rows into `parent`; flatten afterwards.
+ * All three are asynchronous on `stream`. */
+int rvo_join_components(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset,
+                        const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad, float threshold, int64_t id_offset,
+                        int64_t cand_cap, int32_t* parent, int64_t n_labels, uint64_t* hit_count, int32_t* out_overflowed,
+                        void* workspace, size_t workspace_bytes, void* stream);
+int rvo_components_flatten(int32_t* parent, int64_t n, int32_t* labels_out, void* stream);
+int rvo_components_merge(int32_t* parent, const int32_t* labels_src, int64_t n, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Counters for bench.py's `gpu_launches` claim: number of kernels THIS library has launched on the

@@ -621,6 +621,37 @@ class SimpleReverso:
             results_text += f"   📍 Bounding boxes: {it['bbox']} ↔ {it['other_bbox']}\n\n"
         return results_text, items
 
+    def find_recurring_regions(self, similarity_threshold=0.95, max_groups=20):
+        """New: where does an object or scene recur across the loaded database — the groups of regions connected to each other
+        at cosine >= similarity_threshold (single linkage), found on the GPU (`B200VectorDB.find_duplicate_groups`) without
+        listing every pair.  Returns (status text, list of dict{size, members: [dict{filename, bbox}, ...]}) for the
+        `max_groups` largest groups, largest first, members in the database's order."""
+        if not self.vector_db or not self.current_database:
+            return "❌ No database loaded. Please create or load a database first.", []
+        print(f"🔍 Grouping recurring regions of {self.current_database} (threshold={similarity_threshold})")
+        try:
+            with self.vector_db._lock.read():
+                c = self.vector_db._coll(self.current_database)
+                groups = self.vector_db._duplicate_group_rows(self.current_database, similarity_threshold, 2)
+                items = []
+                for g in groups[:max(int(max_groups), 0)]:
+                    members = []
+                    for r in g:
+                        pay = c.payloads[int(r)] or {}
+                        members.append({"filename": pay.get("filename", "Unknown"), "bbox": pay.get("bbox")})
+                    items.append({"size": len(g), "members": members})
+        except Exception as e:
+            return f"❌ Grouping error: {e}", []
+        if not groups:
+            return f"❌ No recurring regions found above threshold {similarity_threshold}", []
+        results_text = f"🎯 Found {len(groups)} groups of recurring regions, showing {len(items)}:\n\n"
+        for i, it in enumerate(items):
+            files = sorted({m["filename"] for m in it["members"]})
+            results_text += f"{i + 1}. {it['size']} regions in {len(files)} images: {', '.join(files[:5])}"
+            results_text += f" (+{len(files) - 5} more)\n" if len(files) > 5 else "\n"
+            results_text += f"   📍 First region: {it['members'][0]['filename']} {it['members'][0]['bbox']}\n\n"
+        return results_text, items
+
     def visualize_detections(self, image, selected_region_index=None):
         """core_system.py:719-757 — rendering, out of scope; returns the image with region boxes drawn."""
         pil = self._to_pil(image).copy()

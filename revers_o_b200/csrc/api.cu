@@ -19,8 +19,10 @@ static std::atomic<long long> opt_select_trace{0};
 size_t selfjoin_workspace_bytes(int d, long long cand_cap);
 int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi, long long q_id_offset, const uint16_t* db,
                     long long n_rows, int d, float threshold, long long id_offset, long long cand_cap, long long* out_pairs,
-                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, int mode,
+                    float* out_scores, long long out_cap, int* parent, unsigned long long* out_count, int* out_overflowed, int mode,
                     bool append, void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream);
+int launch_components_flatten(int* parent, int n, int* labels, int sm_count, cudaStream_t stream);
+int launch_components_merge(int* parent, const int* labels_src, int n, int sm_count, cudaStream_t stream);
 static thread_local char g_err[512] = "";
 std::atomic<long long> g_launches{0};
 std::atomic<long long> g_chain_trace{0};
@@ -860,41 +862,39 @@ int rvo_selfjoin_threshold_ex(const uint16_t* db, int64_t n_rows, int32_t d, int
     int rc = select_device_of(db, &sm);
     if (rc) return rc;
     return launch_selfjoin(db, row_lo, row_hi, id_offset, db, n_rows, d, threshold, id_offset, cand_cap, (long long*)out_pairs,
-                           out_scores, out_cap, (unsigned long long*)out_count, out_overflowed, kJoinTriangle, false, workspace,
+                           out_scores, out_cap, nullptr, (unsigned long long*)out_count, out_overflowed, kJoinTriangle, false, workspace,
                            workspace_bytes, sm, (cudaStream_t)stream);
 }
 
 size_t rvo_join_workspace_bytes(int32_t d, int64_t cand_cap) { return rvo_selfjoin_workspace_bytes_ex(d, cand_cap); }
 
-int rvo_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset, const uint16_t* db,
-                       int64_t n_rows, int32_t d, int64_t d_pad_in, float threshold, int64_t id_offset, int64_t cand_cap,
-                       int64_t* out_pairs, float* out_scores, int64_t out_cap, uint64_t* out_count, int32_t* out_overflowed,
-                       void* workspace, size_t workspace_bytes, void* stream) {
-    DeviceGuard device_guard;
-    RVO_REQUIRE(qdb && db && out_pairs && out_scores && out_count && out_overflowed && workspace, "join: null pointer");
-    RVO_REQUIRE(n_rows > 0 && n_rows < (1ll << 31) && d > 0 && q_row_lo >= 0 && q_row_lo <= q_row_hi && out_cap >= 0 &&
-                    cand_cap > 0,
-                "join: bad shape n_rows=%lld query rows [%lld,%lld)", (long long)n_rows, (long long)q_row_lo,
+// The row-set checks of rvo_join_threshold and rvo_join_components; *triangle: qdb == db with equal id offsets.  Selects the
+// target rows' device and sets *sm to its SM count.
+static int check_join_rows(const char* what, const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset,
+                           const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad_in, int64_t id_offset, int64_t cand_cap,
+                           const void* workspace, bool* triangle, int* sm) {
+    RVO_REQUIRE(n_rows > 0 && n_rows < (1ll << 31) && d > 0 && q_row_lo >= 0 && q_row_lo <= q_row_hi && cand_cap > 0,
+                "%s: bad shape n_rows=%lld query rows [%lld,%lld)", what, (long long)n_rows, (long long)q_row_lo,
                 (long long)q_row_hi);
-    RVO_REQUIRE(d_pad_in == (d + kBlockK - 1) / kBlockK * kBlockK, "join: d_pad must be d rounded up to 64");
+    RVO_REQUIRE(d_pad_in == (d + kBlockK - 1) / kBlockK * kBlockK, "%s: d_pad must be d rounded up to 64", what);
     RVO_REQUIRE(((uintptr_t)workspace & 1023) == 0 && ((uintptr_t)db & 15) == 0 && ((uintptr_t)qdb & 15) == 0,
-                "join: alignment");
-    const bool triangle = qdb == db && q_id_offset == id_offset;
-    if (triangle) {
-        RVO_REQUIRE(q_row_hi <= n_rows, "join: query rows [%lld,%lld) outside the %lld rows of the DB", (long long)q_row_lo,
+                "%s: alignment", what);
+    *triangle = qdb == db && q_id_offset == id_offset;
+    if (*triangle) {
+        RVO_REQUIRE(q_row_hi <= n_rows, "%s: query rows [%lld,%lld) outside the %lld rows of the DB", what, (long long)q_row_lo,
                     (long long)q_row_hi, (long long)n_rows);
     } else {
         // rectangle: the two row sets must be disjoint, by id and in memory (a pair would otherwise be found twice or
         // paired with itself)
-        RVO_REQUIRE(qdb != db, "join: qdb == db with different id offsets");
+        RVO_REQUIRE(qdb != db, "%s: qdb == db with different id offsets", what);
         RVO_REQUIRE(q_id_offset + q_row_hi <= id_offset || id_offset + n_rows <= q_id_offset + q_row_lo,
-                    "join: query ids [%lld,%lld) overlap target ids [%lld,%lld)", (long long)(q_id_offset + q_row_lo),
+                    "%s: query ids [%lld,%lld) overlap target ids [%lld,%lld)", what, (long long)(q_id_offset + q_row_lo),
                     (long long)(q_id_offset + q_row_hi), (long long)id_offset, (long long)(id_offset + n_rows));
         const size_t blk = (size_t)(d_pad_in / kTileCols) * kTileRows * kTileCols;   // bf16 elements per 128-row block
         const uint16_t *q0 = qdb + (size_t)(q_row_lo / kTileRows) * blk,
                        *q1 = qdb + (size_t)((q_row_hi + kTileRows - 1) / kTileRows) * blk,
                        *t1 = db + (size_t)((n_rows + kTileRows - 1) / kTileRows) * blk;
-        RVO_REQUIRE(q_row_lo == q_row_hi || q1 <= db || t1 <= q0, "join: query rows and target rows overlap in memory");
+        RVO_REQUIRE(q_row_lo == q_row_hi || q1 <= db || t1 <= q0, "%s: query rows and target rows overlap in memory", what);
         int qdev = -1, tdev = -1;
         int rc = select_device_of(qdb, nullptr);
         if (rc) return rc;
@@ -902,14 +902,75 @@ int rvo_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, 
         rc = select_device_of(db, nullptr);
         if (rc) return rc;
         RVO_CUDA(cudaGetDevice(&tdev));
-        RVO_REQUIRE(qdev == tdev, "join: query rows on device %d, target rows on device %d", qdev, tdev);
+        RVO_REQUIRE(qdev == tdev, "%s: query rows on device %d, target rows on device %d", what, qdev, tdev);
     }
+    return select_device_of(db, sm);
+}
+
+int rvo_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset, const uint16_t* db,
+                       int64_t n_rows, int32_t d, int64_t d_pad_in, float threshold, int64_t id_offset, int64_t cand_cap,
+                       int64_t* out_pairs, float* out_scores, int64_t out_cap, uint64_t* out_count, int32_t* out_overflowed,
+                       void* workspace, size_t workspace_bytes, void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(qdb && db && out_pairs && out_scores && out_count && out_overflowed && workspace, "join: null pointer");
+    RVO_REQUIRE(out_cap >= 0, "join: out_cap %lld < 0", (long long)out_cap);
+    bool triangle = false;
     int sm = 0;
-    int rc = select_device_of(db, &sm);
+    int rc = check_join_rows("join", qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, d_pad_in, id_offset, cand_cap, workspace,
+                             &triangle, &sm);
     if (rc) return rc;
     return launch_selfjoin(qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, threshold, id_offset, cand_cap,
-                           (long long*)out_pairs, out_scores, out_cap, (unsigned long long*)out_count, out_overflowed,
+                           (long long*)out_pairs, out_scores, out_cap, nullptr, (unsigned long long*)out_count, out_overflowed,
                            triangle ? kJoinTriangle : kJoinRectangle, true, workspace, workspace_bytes, sm, (cudaStream_t)stream);
+}
+
+int rvo_join_components(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset, const uint16_t* db,
+                        int64_t n_rows, int32_t d, int64_t d_pad_in, float threshold, int64_t id_offset, int64_t cand_cap,
+                        int32_t* parent, int64_t n_labels, uint64_t* hit_count, int32_t* out_overflowed, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(qdb && db && parent && hit_count && out_overflowed && workspace, "join components: null pointer");
+    RVO_REQUIRE(n_labels > 0 && n_labels < (1ll << 31), "join components: %lld labels: the forest holds fewer than 2^31 rows",
+                (long long)n_labels);
+    RVO_REQUIRE(q_id_offset + q_row_lo >= 0 && q_id_offset + q_row_hi <= n_labels && id_offset >= 0 && id_offset + n_rows <= n_labels,
+                "join components: query ids [%lld,%lld) or target ids [%lld,%lld) outside the %lld rows of the forest",
+                (long long)(q_id_offset + q_row_lo), (long long)(q_id_offset + q_row_hi), (long long)id_offset,
+                (long long)(id_offset + n_rows), (long long)n_labels);
+    RVO_REQUIRE(((uintptr_t)parent & 3) == 0, "join components: alignment");
+    bool triangle = false;
+    int sm = 0;
+    int rc = check_join_rows("join components", qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, d_pad_in, id_offset,
+                             cand_cap, workspace, &triangle, &sm);
+    if (rc) return rc;
+    int tdev = -1, pdev = -1;
+    RVO_CUDA(cudaGetDevice(&tdev));
+    rc = select_device_of(parent, nullptr);
+    if (rc) return rc;
+    RVO_CUDA(cudaGetDevice(&pdev));
+    RVO_REQUIRE(pdev == tdev, "join components: forest on device %d, target rows on device %d", pdev, tdev);
+    return launch_selfjoin(qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, threshold, id_offset, cand_cap, nullptr, nullptr,
+                           0, parent, (unsigned long long*)hit_count, out_overflowed, triangle ? kJoinTriangle : kJoinRectangle,
+                           true, workspace, workspace_bytes, sm, (cudaStream_t)stream);
+}
+
+int rvo_components_flatten(int32_t* parent, int64_t n, int32_t* labels_out, void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(parent && labels_out, "components flatten: null pointer");
+    RVO_REQUIRE(n > 0 && n < (1ll << 31), "components flatten: n=%lld outside [1, 2^31)", (long long)n);
+    int sm = 0;
+    int rc = select_device_of(parent, &sm);
+    if (rc) return rc;
+    return launch_components_flatten(parent, (int)n, labels_out, sm, (cudaStream_t)stream);
+}
+
+int rvo_components_merge(int32_t* parent, const int32_t* labels_src, int64_t n, void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(parent && labels_src, "components merge: null pointer");
+    RVO_REQUIRE(n > 0 && n < (1ll << 31), "components merge: n=%lld outside [1, 2^31)", (long long)n);
+    int sm = 0;
+    int rc = select_device_of(parent, &sm);
+    if (rc) return rc;
+    return launch_components_merge(parent, labels_src, (int)n, sm, (cudaStream_t)stream);
 }
 
 int rvo_cross_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, int64_t q_id_offset, const uint16_t* db,
@@ -943,7 +1004,7 @@ int rvo_cross_join_threshold(const uint16_t* qdb, int64_t q_row_lo, int64_t q_ro
     RVO_CUDA(cudaGetDevice(&tdev));
     RVO_REQUIRE(qdev == tdev, "cross join: query rows on device %d, target rows on device %d", qdev, tdev);
     return launch_selfjoin(qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, threshold, id_offset, cand_cap,
-                           (long long*)out_pairs, out_scores, out_cap, (unsigned long long*)out_count, out_overflowed,
+                           (long long*)out_pairs, out_scores, out_cap, nullptr, (unsigned long long*)out_count, out_overflowed,
                            query_is_right ? kJoinCrossRight : kJoinCrossLeft, true, workspace, workspace_bytes, sm,
                            (cudaStream_t)stream);
 }

@@ -15,6 +15,10 @@
 //             is stored as (left id, right id) whichever side provides the query rows.
 // The re-score runs the same lanes over the same chunks in the same order in every mode and fmaf is commutative in its two
 // factors, so a pair scores bit-identically whichever of its rows is the query.
+// A hit goes to one of two sinks, a template parameter of pairs_kernel: the pair buffer (append (pair, score)), or, for
+// rvo_join_components (TRIANGLE and RECTANGLE), a lock-free union-find forest over the global rows in which the hit's two rows
+// are unioned.  The union sink gives the connected components of exactly the pair join's edges in O(rows) memory, and stores
+// no pair.
 #include "common.cuh"
 #include "scan_tc.cuh"
 #include "prep_scan_small.cuh"
@@ -49,16 +53,55 @@ __device__ __forceinline__ float dot8(const uint4 a, const uint4 b, float acc) {
     return acc;
 }
 
+// ---- lock-free union-find over global rows (the union sink) ---------------------------------------------------------------------
+// Invariant: parent[x] <= x.  A hook only ever sets the larger of two roots to the smaller (a CAS that requires it to still be a
+// root), and a path-halving store sets a node to its grandparent, which is one of its ancestors; so every path strictly
+// decreases, `find` terminates, and a component's root is its smallest row whatever the order of the hooks.  Other CTAs write
+// the array during the kernel, so it is read with relaxed device-scope loads (never __ldg / the non-coherent path).
+__device__ __forceinline__ int uf_load(const int* p) {
+    int v;
+    asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void uf_store(int* p, int v) {
+    asm volatile("st.relaxed.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ int uf_find(int* parent, int x) {
+    int p = uf_load(parent + x);
+    while (p != x) {
+        const int gp = uf_load(parent + p);
+        if (gp != p) uf_store(parent + x, gp);   // path halving: x skips to its grandparent
+        x = gp;
+        p = uf_load(parent + x);
+    }
+    return x;
+}
+__device__ __forceinline__ void uf_union(int* parent, int a, int b) {
+    for (;;) {
+        a = uf_find(parent, a);
+        b = uf_find(parent, b);
+        if (a == b) return;
+        const int lo = a < b ? a : b, hi = a < b ? b : a;
+        if (atomicCAS(parent + hi, hi, lo) == hi) return;
+        // hi was hooked by another thread in the meantime: retry from the new roots
+    }
+}
+
 // grid (nq), 256 threads: candidates of query row i = row0 + q; 8 lanes per candidate.  j_floor: a candidate j is re-scored
 // when j > j_floor — the query row i in TRIANGLE mode (upper triangle, no self pair), -1 otherwise (every candidate).
-// With gi = i + q_id_offset and gj = j + id_offset a pair is emitted as (min, max) of (gi, gj) in TRIANGLE and RECTANGLE mode,
-// as (gi, gj) in CROSS_LEFT (the query rows are the left collection) and as (gj, gi) in CROSS_RIGHT.
+// With gi = i + q_id_offset and gj = j + id_offset, kUnion == false stores a pair as (min, max) of (gi, gj) in TRIANGLE and
+// RECTANGLE mode, as (gi, gj) in CROSS_LEFT (the query rows are the left collection) and as (gj, gi) in CROSS_RIGHT, keeping the
+// first out_cap; kUnion == true unions gi and gj in `parent` (TRIANGLE and RECTANGLE only) and touches no out_pairs / out_scores.
+// Either way every hit adds to *out_count, one atomic per warp.  The pair instantiation compiles to the code it had before the
+// union sink existed (39 registers, no spills).
+template <bool kUnion>
 __global__ void __launch_bounds__(256) pairs_kernel(const uint4* __restrict__ db, const uint4* __restrict__ qrows, long long row0,
                                                     long long scan_base, int d_pad, const unsigned long long* __restrict__ cand,
                                                     const int* __restrict__ cnt, int cap, float threshold, int mode,
                                                     long long q_id_offset, long long id_offset, long long* __restrict__ out_pairs,
                                                     float* __restrict__ out_scores, long long out_cap,
-                                                    unsigned long long* __restrict__ out_count, int* __restrict__ overflowed) {
+                                                    unsigned long long* __restrict__ out_count, int* __restrict__ overflowed,
+                                                    int* __restrict__ parent) {
     const int q = blockIdx.x;
     const long long i = row0 + q;
     const long long j_floor = mode == kJoinTriangle ? i : -1;
@@ -91,15 +134,19 @@ __global__ void __launch_bounds__(256) pairs_kernel(const uint4* __restrict__ db
             if (bal) {
                 unsigned long long base = 0;
                 if (lane == 0) base = atomicAdd(out_count, (unsigned long long)__popc(bal));
-                base = __shfl_sync(0xFFFFFFFFu, base, 0);
-                if (hit) {
-                    const unsigned long long at = base + __popc(bal & ((1u << lane) - 1u));
-                    if ((long long)at < out_cap) {
-                        const long long gi = i + q_id_offset, gj = j + id_offset;
-                        const bool swap = mode == kJoinCrossRight || (mode < kJoinCrossLeft && gj < gi);
-                        out_pairs[2 * at] = swap ? gj : gi;
-                        out_pairs[2 * at + 1] = swap ? gi : gj;
-                        out_scores[at] = acc;
+                if constexpr (kUnion) {
+                    if (hit) uf_union(parent, (int)(i + q_id_offset), (int)(j + id_offset));
+                } else {
+                    base = __shfl_sync(0xFFFFFFFFu, base, 0);
+                    if (hit) {
+                        const unsigned long long at = base + __popc(bal & ((1u << lane) - 1u));
+                        if ((long long)at < out_cap) {
+                            const long long gi = i + q_id_offset, gj = j + id_offset;
+                            const bool swap = mode == kJoinCrossRight || (mode < kJoinCrossLeft && gj < gi);
+                            out_pairs[2 * at] = swap ? gj : gi;
+                            out_pairs[2 * at + 1] = swap ? gi : gj;
+                            out_scores[at] = acc;
+                        }
                     }
                 }
             }
@@ -148,12 +195,15 @@ size_t selfjoin_workspace_bytes(int d, long long cand_cap) {
 }
 
 // Query rows [q_row_lo, q_row_hi) of `qdb` against the n_rows target rows of `db` in `mode` (JoinMode; the caller has checked
-// what the mode needs: TRIANGLE qdb == db with equal id offsets, RECTANGLE disjoint row sets).  append == false: *out_count and
-// *out_overflowed are reset first (rvo_selfjoin_threshold[_ex]); append == true: pairs are appended at *out_count and overflowed candidate
-// sub-lists are added to *out_overflowed (rvo_join_threshold: every join of a device shares one pair buffer).
+// what the mode needs: TRIANGLE qdb == db with equal id offsets, RECTANGLE disjoint row sets).  parent == nullptr: hits go to
+// the pair buffer (out_pairs, out_scores, out_cap); otherwise they are unioned in the forest `parent` (TRIANGLE or RECTANGLE,
+// every global row of the join < the array's size) and out_pairs / out_scores are not used.  Either way *out_count counts them.
+// append == false: *out_count and *out_overflowed are reset first (rvo_selfjoin_threshold[_ex]); append == true: hits are added
+// at *out_count and overflowed candidate sub-lists are added to *out_overflowed (rvo_join_threshold, rvo_join_components: every
+// join of a device shares one pair buffer or forest).
 int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi, long long q_id_offset, const uint16_t* db,
                     long long n_rows, int d, float threshold, long long id_offset, long long cand_cap, long long* out_pairs,
-                    float* out_scores, long long out_cap, unsigned long long* out_count, int* out_overflowed, int mode,
+                    float* out_scores, long long out_cap, int* parent, unsigned long long* out_count, int* out_overflowed, int mode,
                     bool append, void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream) {
     SelfJoinPlan sp;
     int rc = selfjoin_plan(d, cand_cap, ws, ws_bytes, &sp);
@@ -178,13 +228,43 @@ int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi,
         rc = launch_scan_tc(kModeFilter, db_sub, n_rows - scan_base, 1, sp.d_pad, sp.qb, sp.tc, sp.tau, sp.cand, sp.cnt, sp.cap,
                             nullptr, 0, sm_count, stream);
         if (rc) return rc;
-        pairs_kernel<<<nq, 256, 0, stream>>>((const uint4*)db, (const uint4*)sp.qb, i0, scan_base, sp.d_pad, sp.cand, sp.cnt,
-                                             sp.cap, threshold, mode, q_id_offset, id_offset, out_pairs, out_scores, out_cap,
-                                             out_count, overflowed);
+        (parent ? pairs_kernel<true> : pairs_kernel<false>)<<<nq, 256, 0, stream>>>(
+            (const uint4*)db, (const uint4*)sp.qb, i0, scan_base, sp.d_pad, sp.cand, sp.cnt, sp.cap, threshold, mode, q_id_offset,
+            id_offset, out_pairs, out_scores, out_cap, out_count, overflowed, parent);
         RVO_LAUNCHED();
     }
     if (!append && out_overflowed)
         RVO_CUDA(cudaMemcpyAsync(out_overflowed, sp.overflowed, sizeof(int), cudaMemcpyDeviceToDevice, stream));
+    return RVO_OK;
+}
+
+// labels[x] = root of x (its component's smallest row)
+__global__ void __launch_bounds__(256) components_flatten_kernel(int* parent, int n, int* __restrict__ labels) {
+    for (long long x = blockIdx.x * blockDim.x + threadIdx.x; x < n; x += gridDim.x * blockDim.x) labels[x] = uf_find(parent, (int)x);
+}
+
+// union(x, labels_src[x]) for every x with labels_src[x] != x: folds another forest over the same rows (flattened) into this one
+__global__ void __launch_bounds__(256) components_merge_kernel(int* parent, const int* __restrict__ labels_src, int n) {
+    for (long long x = blockIdx.x * blockDim.x + threadIdx.x; x < n; x += gridDim.x * blockDim.x) {
+        const int l = labels_src[x];
+        if (l != x && l >= 0 && l < n) uf_union(parent, (int)x, l);
+    }
+}
+
+static int components_grid(int n, int sm_count) {
+    const int blocks = (n + 255) / 256, most = (sm_count > 0 ? sm_count : 148) * 8;
+    return blocks < most ? (blocks > 0 ? blocks : 1) : most;
+}
+
+int launch_components_flatten(int* parent, int n, int* labels, int sm_count, cudaStream_t stream) {
+    components_flatten_kernel<<<components_grid(n, sm_count), 256, 0, stream>>>(parent, n, labels);
+    RVO_LAUNCHED();
+    return RVO_OK;
+}
+
+int launch_components_merge(int* parent, const int* labels_src, int n, int sm_count, cudaStream_t stream) {
+    components_merge_kernel<<<components_grid(n, sm_count), 256, 0, stream>>>(parent, labels_src, n);
+    RVO_LAUNCHED();
     return RVO_OK;
 }
 

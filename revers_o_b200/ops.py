@@ -410,6 +410,81 @@ def cross_join_threshold(qdb: torch.Tensor, q_row_lo: int, q_row_hi: int, q_id_o
                                        _stream(dev)), "rvo_cross_join_threshold")
 
 
+def components_out(n_labels: int, device) -> tuple:
+    """Union-find forest of `join_components`: (parent int32 [n_labels] = arange, hit count int64 [1] = 0, overflowed int32 [1]
+    = 0).  Refuses 2^31 rows or more (the forest holds int32 rows)."""
+    if not 0 < n_labels < (1 << 31):
+        raise RvoError(f"duplicate groups need 1 to 2^31 - 1 rows, got {n_labels}")
+    return (torch.arange(n_labels, dtype=torch.int32, device=device), torch.zeros((1,), dtype=torch.int64, device=device),
+            torch.zeros((1,), dtype=torch.int32, device=device))
+
+
+def join_components(qdb: torch.Tensor, q_row_lo: int, q_row_hi: int, q_id_offset: int, db: torch.Tensor, n_rows: int, d: int,
+                    threshold: float, id_offset: int, cand_cap: int, out: tuple) -> None:
+    """rvo_join_components: `join_threshold`'s join (same arguments, same pairs examined), but every pair with cos >= threshold
+    unions its two ids in the forest of `out` (`components_out`, on db's device, indexed by id) instead of being stored.  The
+    hit count and overflow counter are APPENDED to.  Async on the current stream of db's device."""
+    require_cuda(db, "db")
+    require_cuda(qdb, "qdb")
+    for t in (qdb, db):
+        assert t.dtype == torch.bfloat16 and t.dim() == 4 and t.is_contiguous() and t.shape[1] * TILE_COLS == d_pad_of(d)
+    assert n_rows <= db_capacity(db) and q_row_hi <= db_capacity(qdb)
+    parent, hits, over = out
+    assert parent.dtype == torch.int32 and parent.is_contiguous() and parent.device == db.device
+    dev = db.device
+    lib = _lib.load()
+    nbytes = lib.rvo_join_workspace_bytes(d, int(cand_cap))
+    ws = workspace(dev, nbytes)
+    check(lib.rvo_join_components(_ptr(qdb), int(q_row_lo), int(q_row_hi), int(q_id_offset), _ptr(db), int(n_rows), d,
+                                  d_pad_of(d), float(threshold), int(id_offset), int(cand_cap), _ptr(parent), parent.numel(),
+                                  _ptr(hits), _ptr(over), _ptr(ws), nbytes, _stream(dev)), "rvo_join_components")
+
+
+def components_flatten(parent: torch.Tensor) -> torch.Tensor:
+    """rvo_components_flatten: int32 labels [n], label[x] = the smallest row of x's component.  Async."""
+    require_cuda(parent, "parent")
+    assert parent.dtype == torch.int32 and parent.is_contiguous()
+    labels = torch.empty_like(parent)
+    check(_lib.load().rvo_components_flatten(_ptr(parent), parent.numel(), _ptr(labels), _stream(parent.device)),
+          "rvo_components_flatten")
+    return labels
+
+
+def components_merge(parent: torch.Tensor, labels_src: torch.Tensor) -> None:
+    """rvo_components_merge: fold the flattened labels of another forest over the same rows (on parent's device) into
+    `parent`.  Async."""
+    require_cuda(parent, "parent")
+    assert parent.dtype == labels_src.dtype == torch.int32 and parent.is_contiguous() and labels_src.is_contiguous()
+    assert labels_src.shape == parent.shape and labels_src.device == parent.device
+    check(_lib.load().rvo_components_merge(_ptr(parent), _ptr(labels_src), parent.numel(), _stream(parent.device)),
+          "rvo_components_merge")
+
+
+def components_exact(db: torch.Tensor, n_rows: int, d: int, threshold: float, id_offset: int = 0, cand_cap: int = 32768):
+    """Single-linkage groups at a threshold: the connected components of the graph whose edges are exactly the pairs
+    `selfjoin_exact` returns, unioned on the device while the join runs (no pair is stored: O(n_rows) memory).  Returns
+    (labels int64 [n_rows] host array, n_pairs): labels[i] is the smallest id (row + id_offset) of row i's component, and
+    n_pairs the number of pairs with cos >= threshold.  Overflow protocol of `selfjoin_exact`: overflowed candidate lists re-run
+    the join with 8x the capacity (exact once cand_cap >= n_rows + 4096), keeping the forest (re-applying an edge changes
+    nothing) and resetting the hit count.  Synchronises."""
+    require_cuda(db, "db")
+    assert db.dtype == torch.bfloat16 and db.dim() == 4 and db.is_contiguous()
+    parent, hits, over = components_out(n_rows, db.device)
+    cap = int(cand_cap)
+    while True:
+        hits.zero_()
+        over.zero_()
+        join_components(db, 0, n_rows, 0, db, n_rows, d, threshold, 0, cap, (parent, hits, over))
+        m, ov = int(hits.item()), int(over.item())
+        if ov > 0 and cap < n_rows + 4096:
+            cap = min(cap * 8, n_rows + 4096 + TILE_ROWS * 16)
+            continue
+        if ov > 0:
+            raise RvoError(f"self-join candidate lists overflowed at capacity {cap} for {n_rows} rows")
+        labels = components_flatten(parent).cpu().numpy().astype("int64")
+        return labels + int(id_offset), m
+
+
 def merge_topk(ids: torch.Tensor, scores: torch.Tensor, counts: torch.Tensor, k: int):
     """K3.  ids int64 [G,nq,k], scores f32 [G,nq,k], counts int32 [G,nq] -> merged (ids, scores, counts)."""
     require_cuda(ids, "ids")

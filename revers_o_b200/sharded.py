@@ -12,7 +12,8 @@ product path.
 The self-join of a collection row-sharded over the devices of ONE process (B200VectorDB(devices=[...]).find_near_duplicates) is
 here too: `selfjoin_plan` (pure host logic) and `selfjoin_sharded`, which joins the shards where they live and moves only
 query blocks.  So is the join between two such collections (B200VectorDB.join_collections): `crossjoin_plan` and
-`crossjoin_sharded`, run by the same device loop.
+`crossjoin_sharded`, run by the same device loop, and the duplicate groups of a row-sharded collection
+(B200VectorDB.find_duplicate_groups): `components_sharded`, the self-join's items unioned into one forest per device.
 """
 from __future__ import annotations
 
@@ -218,23 +219,52 @@ def crossjoin_sharded(left: list, right: list, d: int, threshold: float, max_pai
     return _join_on_devices(list(left) + list(right), items, d, threshold, max_pairs, cand_cap, block, device_ms, len(left))
 
 
+def components_sharded(shards: list, d: int, threshold: float, cand_cap: int = 32768, block: int = 4096,
+                       device_ms: dict | None = None):
+    """Single-linkage groups of a collection row-sharded over the devices of one process: the connected components of exactly
+    the pairs `selfjoin_sharded` returns.  shards as there.  Each device runs its `selfjoin_plan` items into a union-find forest
+    over all the global rows (`rvo_join_components`); then every other device's forest is flattened, copied to the first device
+    and merged there (`rvo_components_merge`), so every edge any device found is in the result.  Returns (labels int64 [N] host
+    array over the global rows [0, N), N = the end of the last shard, each the smallest global row of its component; n_pairs) —
+    the same as `ops.components_exact` on one device."""
+    sizes = [int(n) for _, n, _ in shards]
+    plan = selfjoin_plan(sizes, block)
+    items: dict[int, list[JoinItem]] = {}
+    for g, its in enumerate(plan):
+        items.setdefault(shards[g][0].device.index, []).extend(its)
+    n_labels = max(int(r0) + int(n) for _, n, r0 in shards)
+    done = _join_on_devices(shards, items, d, threshold, 0, cand_cap, block, device_ms, None, n_labels)
+    devs = sorted(done)
+    root = done[devs[0]][0]
+    for dv in devs[1:]:
+        labels = ops.components_flatten(done[dv][0])
+        with torch.cuda.device(root.device):
+            ops.components_merge(root, labels.to(root.device))    # a peer copy, ordered after the flatten and before the merge
+    labels = ops.components_flatten(root).cpu().numpy().astype(np.int64)
+    return labels, sum(m for _, m in done.values())
+
+
 def _join_on_devices(shards: list, items: dict, d: int, threshold: float, max_pairs: int, cand_cap: int, block: int,
-                     device_ms: dict | None, n_left: int | None):
+                     device_ms: dict | None, n_left: int | None, n_labels: int | None = None):
     """Run {device index: [JoinItem]} over shards [(tiled storage, rows, first global row)].  n_left None: the items are a
     self-join's (triangles and rectangles, `rvo_join_threshold`); otherwise shards [0, n_left) are the left collection and
-    the rest the right one, and every item is a cross join (`rvo_cross_join_threshold`).
+    the rest the right one, and every item is a cross join (`rvo_cross_join_threshold`).  n_labels given (a self-join only): the
+    pairs are not stored but unioned into one forest per device over the n_labels global rows (`rvo_join_components`), and
+    {device index: (parent int32 [n_labels] on that device, pairs found there)} is returned.
 
     Every item is enqueued, round-robin over the devices, before any synchronisation: one host sync per device.  A query
     block of another device is copied (a peer copy) into one of two staging blocks on the target device, ordered after the
     source device's current stream; the joins run on each device's current stream and append to one pair buffer per device.
     Overflow protocol of `ops.selfjoin_exact`, judged per device: overflowed candidate lists re-run that device's items with
     8x the capacity (exact once it covers the rows scanned + 4096), a pair count above the buffer re-runs them with a buffer
-    of that count.  `device_ms`: filled with each device's busy time (CUDA events, ms) of the last attempt."""
+    of that count (pair buffers only: a forest keeps its edges across a re-run, since re-applying an edge changes nothing).
+    `device_ms`: filled with each device's busy time (CUDA events, ms) of the last attempt."""
     cap = {dv: int(cand_cap) for dv in items}
     out_cap = {dv: int(max_pairs) for dv in items}
     rows_scanned = {dv: max(it.t_hi - it.t_lo for it in its) for dv, its in items.items() if its}
     todo = sorted(rows_scanned)
     done: dict[int, tuple] = {}
+    forests = {dv: ops.components_out(n_labels, torch.device("cuda", dv))[0] for dv in todo} if n_labels else {}
     while todo:
         ready = {}           # copies read a shard after what its device's current stream had queued before the join
         for v, _, _ in shards:
@@ -242,7 +272,7 @@ def _join_on_devices(shards: list, items: dict, d: int, threshold: float, max_pa
                 ready[v.device.index] = torch.cuda.Event()
                 ready[v.device.index].record(torch.cuda.current_stream(v.device))
         runs = {dv: _join_runs(items[dv], shards, dv) for dv in todo}
-        st = {dv: _JoinState(torch.device("cuda", dv), out_cap[dv], d, block, ready, n_left) for dv in todo}
+        st = {dv: _JoinState(torch.device("cuda", dv), out_cap[dv], d, block, ready, n_left, forests.get(dv)) for dv in todo}
         for k in range(max(len(r) for r in runs.values())):
             for dv in todo:
                 if k < len(runs[dv]):
@@ -254,20 +284,24 @@ def _join_on_devices(shards: list, items: dict, d: int, threshold: float, max_pa
             torch.cuda.current_stream(s.dev).synchronize()
             if device_ms is not None:
                 device_ms[dv] = s.start.elapsed_time(s.stop)
-            pairs, scores, count, over = s.out
+            count, over = s.out[-2:]
             m, ov = int(count.item()), int(over.item())
             if ov > 0 and cap[dv] < rows_scanned[dv] + 4096:
                 cap[dv] = min(cap[dv] * 8, rows_scanned[dv] + 4096 + ops.TILE_ROWS * 16)
                 retry.append(dv)
-            elif m > out_cap[dv]:
+            elif not n_labels and m > out_cap[dv]:
                 out_cap[dv] = m
                 retry.append(dv)
             elif ov > 0:
                 what = "self-join" if n_left is None else "cross join"
                 raise _lib.RvoError(f"{what} candidate lists overflowed at capacity {cap[dv]} on cuda:{dv}")
+            elif n_labels:
+                done[dv] = (s.out[0], m)
             else:
-                done[dv] = (pairs[:m].cpu().numpy(), scores[:m].cpu().numpy())
+                done[dv] = (s.out[0][:m].cpu().numpy(), s.out[1][:m].cpu().numpy())
         todo = retry
+    if n_labels:
+        return done
     if not done:
         return np.zeros((0, 2), np.int64), np.zeros(0, np.float32)
     return np.concatenate([done[dv][0] for dv in sorted(done)]), np.concatenate([done[dv][1] for dv in sorted(done)])
@@ -290,11 +324,16 @@ def _join_runs(its: list[JoinItem], shards: list, dv: int) -> list[JoinItem]:
 
 
 class _JoinState:
-    """Pair buffer, staging blocks and streams of one device during `_join_on_devices`."""
+    """Output (a pair buffer, or a union-find forest), staging blocks and streams of one device during `_join_on_devices`."""
 
-    def __init__(self, dev: torch.device, out_cap: int, d: int, block: int, ready: dict, n_left: int | None = None):
+    def __init__(self, dev: torch.device, out_cap: int, d: int, block: int, ready: dict, n_left: int | None = None,
+                 parent: torch.Tensor | None = None):
         self.dev, self.ready, self.n_left = dev, ready, n_left
-        self.out = ops.join_out(out_cap, dev)
+        if parent is None:
+            self.out, self.join = ops.join_out(out_cap, dev), ops.join_threshold
+        else:       # the forest of earlier attempts is kept; the hit count and overflow counter start at 0
+            self.out = (parent, torch.zeros((1,), dtype=torch.int64, device=dev), torch.zeros((1,), dtype=torch.int32, device=dev))
+            self.join = ops.join_components
         self.d, self.block = d, block
         self.slots: list = []                    # two staging blocks: the copy of one overlaps the join of the other
         self.free: list = []                     # event per slot: the join that last read it has finished
@@ -310,7 +349,7 @@ class _JoinState:
         cur = torch.cuda.current_stream(self.dev)
         if it.q_shard == it.t_shard:
             with torch.cuda.device(self.dev):
-                ops.join_threshold(tv, it.q_lo, it.q_hi, t_row0, tv, it.t_hi, d, threshold, t_row0, cand_cap, self.out)
+                self.join(tv, it.q_lo, it.q_hi, t_row0, tv, it.t_hi, d, threshold, t_row0, cand_cap, self.out)
             return
         target = tv[it.t_lo // ops.TILE_ROWS:]
         if qv.device == self.dev:
@@ -336,8 +375,7 @@ class _JoinState:
             qdb, q_lo, q_hi, q_off = self.slots[k], it.q_lo - b0 * ops.TILE_ROWS, it.q_hi - b0 * ops.TILE_ROWS, q_row0 + b0 * ops.TILE_ROWS
         with torch.cuda.device(self.dev):
             if self.n_left is None:
-                ops.join_threshold(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo, cand_cap,
-                                   self.out)
+                self.join(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo, cand_cap, self.out)
             else:
                 ops.cross_join_threshold(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo,
                                          it.q_shard >= self.n_left, cand_cap, self.out)

@@ -8,7 +8,8 @@ It duck-types exactly the five qdrant-client methods core_system.py uses (SURVEY
   .search(collection_name, query_vector, limit, score_threshold) -> [obj(.score,.payload)]     :659-664
 plus the batched entry point `search_batch` (new; reduces to `search` row by row, SURVEY.md F7), and two threshold joins
 (new): `find_near_duplicates` (every pair within one collection at cos >= threshold) and `join_collections` (every pair across
-two collections, possibly of two B200VectorDB instances: which regions of one archive also appear in another).
+two collections, possibly of two B200VectorDB instances: which regions of one archive also appear in another), and the groups
+of the first (new): `find_duplicate_groups` (the connected components of those pairs, unioned on the GPU, no pair stored).
 
 Vectors live on the GPU(s) as L2-normalised bf16 rows in the TILED storage of include/revers_o_b200.h
 ([row/128][col/64][128][64]: one contiguous 16 KiB TMA box per tile; the DB is DEFINED as its bf16 values).  All arithmetic
@@ -708,6 +709,32 @@ class B200VectorDB:
             p, sc = ops.selfjoin_exact(vectors, n, c.dim, threshold, max_pairs=max_pairs, id_offset=s.row0)
             return [(c.ids[int(a)], c.ids[int(b)]) for a, b in p], sc
 
+    def find_duplicate_groups(self, collection_name: str, threshold: float = 0.95, min_size: int = 2) -> list:
+        """Single-linkage groups at a cosine threshold: the connected components of the graph whose edges are exactly the pairs
+        `find_near_duplicates(collection_name, threshold)` returns — "where does this object or scene recur across my
+        archive?".  The edges are unioned on the GPU while the join runs (`ops.components_exact`, or `sharded.components_sharded`
+        for a row-sharded collection), so memory grows with the rows, not with the pairs: a static scene of m identical frames
+        costs m labels, not m(m-1)/2 pairs.  Returns a list of groups, each a list of point ids in row order; the largest group
+        first, groups of equal size by their first row.  Groups smaller than `min_size` are left out (min_size=1 keeps
+        the singletons).  An empty collection, or one with a single point, has no groups."""
+        with self._lock.read():
+            return [[self._coll(collection_name).ids[r] for r in g]
+                    for g in self._duplicate_group_rows(collection_name, threshold, min_size)]
+
+    def _duplicate_group_rows(self, collection_name: str, threshold: float, min_size: int) -> list:
+        """`find_duplicate_groups` in global rows; the caller holds the read lock."""
+        c = self._coll(collection_name)
+        active = [s for s in c.shards if s.n]
+        if sum(s.n for s in active) < 2:
+            return []
+        if len(active) > 1:
+            from .sharded import components_sharded
+            labels, _ = components_sharded([(s.vectors, s.n, s.row0) for s in active], c.dim, threshold)
+            return group_labels(labels, min_size)
+        s = active[0]
+        labels, _ = ops.components_exact(s.vectors, s.n, c.dim, threshold, id_offset=s.row0)
+        return group_labels(labels, min_size, row0=s.row0)
+
     def join_collections(self, collection_name: str, other_collection_name: str, threshold: float = 0.95,
                          max_pairs: int = 1 << 22, other: B200VectorDB | None = None):
         """All pairs (point of `collection_name`, point of `other_collection_name`) with cosine >= threshold: "which regions of
@@ -1014,6 +1041,22 @@ class B200VectorDB:
             with torch.cuda.device(s.device):
                 ops.normalize_rows(src[i:j], db=s.vectors, row0=r)
             i = j
+
+
+def group_labels(labels, min_size: int = 2, row0: int = 0) -> list:
+    """Component labels -> groups.  labels[i] is the component of row row0 + i (equal labels, equal component).  Returns the
+    groups of at least `min_size` rows (at least 1) as lists of rows, each in row order; the largest group first, groups of
+    equal size ordered by their smallest row."""
+    labels = np.asarray(labels, dtype=np.int64)
+    if labels.size == 0:
+        return []
+    order = np.argsort(labels, kind="stable")            # rows of one label together, in row order
+    sl = labels[order]
+    starts = np.flatnonzero(np.r_[True, sl[1:] != sl[:-1]])
+    sizes = np.diff(np.r_[starts, sl.size])
+    keep = np.flatnonzero(sizes >= max(int(min_size), 1))
+    keep = keep[np.lexsort((order[starts[keep]], -sizes[keep]))]
+    return [(order[starts[k]: starts[k] + sizes[k]] + row0).tolist() for k in keep]
 
 
 def _copy_blocks_to_device(view: np.ndarray, dst: torch.Tensor, chunk_blocks: int = 4096) -> None:
