@@ -341,6 +341,40 @@ int rvo_components_flatten(int32_t* parent, int64_t n, int32_t* labels_out, void
 int rvo_components_merge(int32_t* parent, const int32_t* labels_src, int64_t n, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * k-nearest-neighbour join: for every query row, in order, the k stored rows of `db` with the highest score — K2 with stored
+ * rows as its queries.  No reference counterpart (the reference searches one embedded query at a time).
+ *   qdb        [dev] tiled bf16 storage holding the query rows; their ids are row + q_id_offset
+ *   q_rows     [dev] int64 or NULL: NULL, the query rows are [q_row_lo, q_row_hi); otherwise they are q_rows[q_row_lo ..
+ *              q_row_hi) (rows of qdb's capacity)
+ *   db         [dev] tiled bf16 storage of the n_rows target rows (may be qdb itself, and may be empty); ids row + id_offset
+ *   score      the fp32 dot of the two stored bf16 rows; the query row is NOT re-normalised.  It equals the threshold joins'
+ *              score of the same pair up to fp32 summation order.
+ *   k          1..RVO_MAX_K, 1..RVO_MAX_K - 1 with exclude_self
+ *   score_threshold   hits with score < threshold are dropped (== is kept); -INFINITY for none
+ *   exclude_self      1 (self mode: qdb and db are one collection): the query row's own id never appears in its list, its
+ *              exact copies do.  The search keeps k + 1 per row and drops the own id when present, else the last entry.
+ *   path       RVO_PATH_AUTO: tcgen05 scan for every block of query rows (option "knn_block", default 8192; tails of <= 4
+ *              rows included), fused select
+ *              and fp32 re-score.  RVO_PATH_SMALL / RVO_PATH_DENSE: the fp32 overflow routes, for at most RVO_SMALL_Q rows
+ *              given as a q_rows list (d_pad <= 2048).
+ *   out_ids / out_scores / out_counts   as rvo_search_topk, row q for query row q_row_lo + q: [nq, k] ids (score descending,
+ *              ties by lower id, -1 pad), scores (-inf pad), counts [nq] (0..k, or -1: the query overflowed the fused path's
+ *              candidate lists, re-run it with path SMALL, then DENSE, exactly as rvo_search_topk's flagged queries)
+ *   workspace  [dev] rvo_knn_workspace_bytes(n_rows, d, nq, k, path) bytes with nq = q_row_hi - q_row_lo, 1024-B aligned
+ * qdb, db and the workspace must be on one device.  Asynchronous on `stream`.
+ * rvo_knn_exclude_self: the self mode's exclusion on its own, for lists of k + 1 merged across shards (rvo_merge_topk):
+ * ids/scores [nq, k + 1], counts [nq] -> out_* [nq, k]; query q's own id is q_id_offset + (q_rows ? q_rows[q] : q_row_lo + q).
+ * ---------------------------------------------------------------------------------------------- */
+size_t rvo_knn_workspace_bytes(int64_t n_rows, int32_t d, int32_t nq, int32_t k, int32_t path);
+int rvo_knn_join(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, const int64_t* q_rows, int64_t q_id_offset,
+                 const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad, int32_t k, float score_threshold,
+                 int64_t id_offset, int32_t exclude_self, int32_t path, int64_t* out_ids, float* out_scores,
+                 int32_t* out_counts, void* workspace, size_t workspace_bytes, void* stream);
+int rvo_knn_exclude_self(const int64_t* ids, const float* scores, const int32_t* counts, int32_t nq, int32_t k,
+                         int64_t q_row_lo, const int64_t* q_rows, int64_t q_id_offset, int64_t* out_ids, float* out_scores,
+                         int32_t* out_counts, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Counters for bench.py's `gpu_launches` claim: number of kernels THIS library has launched on the
  * calling process since load (monotonic).
  * ---------------------------------------------------------------------------------------------- */
@@ -360,6 +394,7 @@ float rvo_last_scan_ms(void);
  *         0: general select only), "exchange_timeout_ms" (peer-exchange wait limit, default 60000),
  *         "seed_max" (1 default: the seed scan writes one maximum per 32 sample rows; 0: every score),
  *         "pdl" (programmatic dependent launch along the search chain: 0 default off, 2 tensor-path chain, 1 also the Q <= 4 chain),
+ *         "knn_block" (query rows per search block of rvo_knn_join, 256..16384, default 8192; rvo_knn_workspace_bytes follows it),
  *         debugging (value = a device pointer the caller owns, 0 = off): "chain_trace" (u64 [8][2]: earliest start / latest end
  *         of normalise, seed scan, seed threshold, scan, select on %globaltimer; initialise to (UINT64_MAX, 0) pairs),
  *         "select_trace" (u64 [nq][16] phase stamps of the last-level select), "merge_trace" (u64 [3]), "pool_trace".        */

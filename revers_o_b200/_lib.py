@@ -82,6 +82,12 @@ PROTOTYPES = {
                                       C.c_void_p, C.c_size_t, C.c_void_p]),
     "rvo_components_flatten": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "rvo_components_merge": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "rvo_knn_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
+    "rvo_knn_join": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32,
+                               C.c_int64, C.c_int32, C.c_float, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                               C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rvo_knn_exclude_self": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_void_p,
+                                       C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rvo_kernel_launch_count": (C.c_int64, []),
     "rvo_last_scan_ms": (C.c_float, []),
     "rvo_set_option": (C.c_int, [C.c_char_p, C.c_int64]),

@@ -621,6 +621,57 @@ class SimpleReverso:
             results_text += f"   📍 Bounding boxes: {it['bbox']} ↔ {it['other_bbox']}\n\n"
         return results_text, items
 
+    def find_best_matches(self, other_database_name, similarity_threshold=0.0, max_results=20):
+        """New: one-to-one correspondences between the loaded database and another one — the pairs of regions that are each
+        other's best match (mutual nearest neighbours) at cosine >= similarity_threshold, from two k = 1 joins on the GPU
+        (`B200VectorDB.knn_join`, this database against the other and back; `vector_db.mutual_best`).  The other database is
+        opened and checked as `find_shared_regions` does.  Returns (status text, list of dict{score, filename, bbox,
+        other_filename, other_bbox}) for the `max_results` best pairs: score descending, ties by the loaded database's row,
+        then the other database's row."""
+        from .vector_db import mutual_best
+        if not self.vector_db or not self.current_database:
+            return "❌ No database loaded. Please create or load a database first.", []
+        if not other_database_name:
+            return "❌ Please provide a database name", []
+        db_path = f"{self.db_root}/{other_database_name}"
+        if not os.path.exists(db_path):
+            return f"❌ Database not found: {other_database_name}", []
+        if self.vector_db.path and os.path.realpath(self.vector_db.path) == os.path.realpath(db_path):
+            return f"❌ {other_database_name} is the loaded database: choose another database to compare with", []
+        other = None
+        try:
+            other = self._new_client(db_path)
+            collection_name = f"{COLLECTION_PREFIX}{other_database_name}"
+            names = [c.name for c in other.get_collections().collections]
+            if collection_name not in names:
+                if other_database_name in names:  # legacy naming, as in load_database
+                    collection_name = other_database_name
+                else:
+                    return f"❌ Collection not found in database: {other_database_name}", []
+            print(f"🔍 Matching {self.current_database} with {collection_name} (threshold={similarity_threshold})")
+            with self.vector_db._read_both(other):
+                r_ab, s_ab, c_ab = self.vector_db._knn_rows(self.current_database, 1, similarity_threshold, collection_name, other)
+                r_ba, _, c_ba = other._knn_rows(collection_name, 1, similarity_threshold, self.current_database, self.vector_db)
+                pairs, scores = mutual_best(r_ab, c_ab, r_ba, c_ba, s_ab)
+                a, b = self.vector_db._coll(self.current_database), other._coll(collection_name)
+                items = []
+                for (i, j), s in zip(pairs[:max(int(max_results), 0)].tolist(), scores.tolist()):
+                    pa, pb = a.payloads[int(i)] or {}, b.payloads[int(j)] or {}
+                    items.append({"score": float(s), "filename": pa.get("filename", "Unknown"), "bbox": pa.get("bbox"),
+                                  "other_filename": pb.get("filename", "Unknown"), "other_bbox": pb.get("bbox")})
+        except Exception as e:
+            return f"❌ Match error: {e}", []
+        finally:
+            if other is not None:
+                other.close()
+        if len(pairs) == 0:
+            return f"❌ No mutual best matches found above threshold {similarity_threshold}", []
+        results_text = f"🎯 Found {len(pairs)} one-to-one matches with {other_database_name}, showing {len(items)}:\n\n"
+        for i, it in enumerate(items):
+            results_text += f"{i + 1}. {it['filename']} ↔ {it['other_filename']} (Similarity: {it['score']:.3f})\n"
+            results_text += f"   📍 Bounding boxes: {it['bbox']} ↔ {it['other_bbox']}\n\n"
+        return results_text, items
+
     def find_recurring_regions(self, similarity_threshold=0.95, max_groups=20):
         """New: where does an object or scene recur across the loaded database — the groups of regions connected to each other
         at cosine >= similarity_threshold (single linkage), found on the GPU (`B200VectorDB.find_duplicate_groups`) without

@@ -23,6 +23,11 @@ int launch_selfjoin(const uint16_t* qdb, long long q_row_lo, long long q_row_hi,
                     bool append, void* ws, size_t ws_bytes, int sm_count, cudaStream_t stream);
 int launch_components_flatten(int* parent, int n, int* labels, int sm_count, cudaStream_t stream);
 int launch_components_merge(int* parent, const int* labels_src, int n, int sm_count, cudaStream_t stream);
+int launch_knn_intake(const uint16_t* qdb, long long row0, const int64_t* rows, int nq, int n_pad_rows, int d_pad, uint16_t* qb,
+                      float* qn, float* margin, void* zero_base, size_t zero_bytes, cudaStream_t stream);
+int launch_knn_exclude(const int64_t* ids, const float* scores, const int32_t* counts, int nq, int k, long long row0,
+                       const int64_t* rows, long long q_id_offset, int64_t* out_ids, float* out_scores, int32_t* out_counts,
+                       cudaStream_t stream);
 static thread_local char g_err[512] = "";
 std::atomic<long long> g_launches{0};
 std::atomic<long long> g_chain_trace{0};
@@ -35,7 +40,8 @@ void set_error(const char* fmt, ...) {
     va_end(ap);
 }
 
-static std::atomic<long long> opt_force_path{0}, opt_m_sub{0}, opt_cand_cap{32768}, opt_final_ratio{48}, opt_time_scan{0}, opt_hot{1}, opt_seed_max{1};
+static std::atomic<long long> opt_force_path{0}, opt_m_sub{0}, opt_cand_cap{32768}, opt_final_ratio{48}, opt_time_scan{0}, opt_hot{1}, opt_seed_max{1},
+    opt_knn_block{8192};
 static cudaEvent_t g_ev0 = nullptr, g_ev1 = nullptr;
 static bool g_ev_valid = false;
 
@@ -281,6 +287,15 @@ static int prep_queries(const SearchPlan& sp, const float* queries, int nq, int 
                                  (void*)sp.cnt, sp.cnt_bytes);
 }
 
+// Stored rows as the queries of a search (rvo_knn_join): query q is row (rows ? rows[q] : row0 + q) of the tiled storage qdb,
+// on the searched rows' device.  It replaces the normalise launch: knn.cu's intake writes the query operand, its fp32 copy,
+// the margins and the cleared counters in one launch.
+struct StoredQueries {
+    const uint16_t* qdb;
+    long long row0;
+    const int64_t* rows;
+};
+
 }  // namespace rvo
 
 using namespace rvo;
@@ -319,6 +334,10 @@ int rvo_set_option(const char* name, int64_t value) {
     else if (!strcmp(name, "time_scan")) opt_time_scan = value;
     else if (!strcmp(name, "hot")) opt_hot = value;
     else if (!strcmp(name, "seed_max")) opt_seed_max = value;
+    else if (!strcmp(name, "knn_block")) {
+        RVO_REQUIRE(value >= 256 && value <= 16384, "option knn_block=%lld outside 256..16384", (long long)value);
+        opt_knn_block = value;
+    }
     else if (!strcmp(name, "exchange_timeout_ms")) g_exchange_timeout_ms = value > 0 ? value : 1;
     else if (!strcmp(name, "merge_trace")) g_merge_trace = value;
     else if (!strcmp(name, "pool_path")) g_force_cuda_core_pool = value == 1;
@@ -413,11 +432,11 @@ size_t rvo_search_workspace_bytes_ex(int64_t n_rows, int32_t d, int32_t nq, int3
 static int search_impl(const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad_in, const float* queries, int32_t nq,
                        int32_t k, float score_threshold, int64_t id_offset, int64_t* out_ids, float* out_scores,
                        int32_t* out_counts, void* workspace, size_t workspace_bytes, void* stream_, const PushArgs* push,
-                       int path = RVO_PATH_AUTO) {
+                       int path = RVO_PATH_AUTO, const StoredQueries* stored = nullptr) {
     DeviceGuard device_guard;
     RVO_REQUIRE(path >= RVO_PATH_AUTO && path <= RVO_PATH_DENSE, "search_topk: path %d (0 auto, 1 fp32 scan, 2 tcgen05, 3 dense fp32)", path);
     cudaStream_t stream = (cudaStream_t)stream_;
-    RVO_REQUIRE(queries && out_ids && out_scores && out_counts && workspace, "search_topk: null pointer");
+    RVO_REQUIRE((queries || stored) && out_ids && out_scores && out_counts && workspace, "search_topk: null pointer");
     RVO_REQUIRE(n_rows >= 0 && d > 0 && nq > 0, "search_topk: bad shape n_rows=%lld d=%d nq=%d", (long long)n_rows, d, nq);
     RVO_REQUIRE(k >= 1 && k <= RVO_MAX_K, "search_topk: k=%d outside 1..%d", k, RVO_MAX_K);
     RVO_REQUIRE(n_rows == 0 || db, "search_topk: null db");
@@ -490,8 +509,17 @@ static int search_impl(const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_
             sa.zero_base = (uint4*)sp.cnt;
             sa.zero_u4 = (long long)(sp.cnt_bytes / 16);
         }
+        if (stored) {
+            // the fp32 scan reads the stored rows' fp32 copy instead of normalising raw queries; the intake also clears the
+            // FILTER pass's counters, which only the normalising scan would otherwise clear
+            rc = launch_knn_intake(stored->qdb, stored->row0, stored->rows, nq, RVO_SMALL_Q, sp.d_pad, nullptr, sp.qn, nullptr,
+                                   (void*)sp.cnt, sp.cnt_bytes, stream);
+            if (rc) return rc;
+            sa.q = sp.qn;
+            sa.q_ld = sp.d_pad;
+        }
         if (!sampled && (rc = scan_timer(true, stream))) return rc;
-        rc = launch_scan_small(sa, true, true, sm, stream);
+        rc = launch_scan_small(sa, true, !stored, sm, stream);
         if (rc) return rc;
         if (!sampled && (rc = scan_timer(false, stream))) return rc;
         DenseTopkArgs da;
@@ -531,7 +559,9 @@ static int search_impl(const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_
         sl.score_floor = score_threshold;
         return launch_select_final(sl, fa, nq, stream);     // a sub-list that overflowed flags the query (-1): path DENSE serves it
     }
-    rc = prep_queries(sp, queries, nq, d, stream);
+    rc = stored ? launch_knn_intake(stored->qdb, stored->row0, stored->rows, nq, sp.tc.nq_pad, sp.d_pad, sp.qb, sp.qn, sp.margin,
+                                    (void*)sp.cnt, sp.cnt_bytes, stream)
+                : prep_queries(sp, queries, nq, d, stream);
     if (rc) return rc;
 
     const int nq_pad = sp.tc.nq_pad;
@@ -633,6 +663,127 @@ int rvo_search_topk_ex(const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_
                        int32_t* out_counts, void* workspace, size_t workspace_bytes, void* stream) {
     return search_impl(db, n_rows, d, d_pad, queries, nq, k, score_threshold, id_offset, out_ids, out_scores, out_counts,
                        workspace, workspace_bytes, stream, nullptr, path);
+}
+
+// ---- k-nearest-neighbour join (knn.cu) --------------------------------------------------------------------------------
+// Query blocks of option "knn_block" stored rows (default 8192), each one K2 search.  The block's candidate lists dominate the
+// workspace (3.3 GB at 8192 rows, d = 1024).  Measured on the 2M x 1024 self kNN at k = 10 (scripts/bench_knn_join.py, DESIGN.md
+// §4): larger blocks stream each DB tile for more queries; 8192 rows beat 4096 by ~3 % for twice the workspace.
+
+struct KnnLayout {
+    int block, kk, search_path;
+    size_t search_bytes, lists_off, scores_off, counts_off, bytes;
+};
+
+// Workspace of rvo_knn_join: one block's search workspace, then (self mode) the block's [block][k+1] lists before exclusion.
+// Sized for k + 1 lists whichever the mode, so that one size serves both.
+static bool knn_layout(int64_t n_rows, int32_t d, int64_t nq, int32_t k, int32_t path, KnnLayout* L) {
+    if (n_rows < 0 || d <= 0 || nq <= 0 || k <= 0 || k > RVO_MAX_K || path < RVO_PATH_AUTO || path > RVO_PATH_DENSE) return false;
+    const long long block = opt_knn_block.load();
+    L->block = (int)(nq < block ? nq : block);
+    L->kk = k < RVO_MAX_K ? k + 1 : k;
+    L->search_path = path == RVO_PATH_AUTO ? RVO_PATH_TENSOR : path;   // AUTO: tcgen05 for every block, tails of <= 4 rows too
+    SearchPlan sp;
+    if (make_plan(n_rows, d, L->block, L->kk, L->search_path, nullptr, 0, &sp)) return false;
+    L->search_bytes = sp.bytes;
+    L->lists_off = align_up(L->search_bytes, 256);
+    L->scores_off = L->lists_off + align_up((size_t)L->block * L->kk * 8, 256);
+    L->counts_off = L->scores_off + align_up((size_t)L->block * L->kk * 4, 256);
+    L->bytes = L->counts_off + align_up((size_t)L->block * 4, 256);
+    return true;
+}
+
+size_t rvo_knn_workspace_bytes(int64_t n_rows, int32_t d, int32_t nq, int32_t k, int32_t path) {
+    KnnLayout L;
+    return knn_layout(n_rows, d, nq, k, path, &L) ? L.bytes : 0;
+}
+
+int rvo_knn_join(const uint16_t* qdb, int64_t q_row_lo, int64_t q_row_hi, const int64_t* q_rows, int64_t q_id_offset,
+                 const uint16_t* db, int64_t n_rows, int32_t d, int64_t d_pad_in, int32_t k, float score_threshold, int64_t id_offset,
+                 int32_t exclude_self, int32_t path, int64_t* out_ids, float* out_scores, int32_t* out_counts, void* workspace,
+                 size_t workspace_bytes, void* stream_) {
+    DeviceGuard device_guard;
+    cudaStream_t stream = (cudaStream_t)stream_;
+    RVO_REQUIRE(qdb && out_ids && out_scores && out_counts && workspace, "knn join: null pointer");
+    RVO_REQUIRE(n_rows == 0 || db, "knn join: null db");
+    RVO_REQUIRE(exclude_self == 0 || exclude_self == 1, "knn join: exclude_self must be 0 or 1, got %d", (int)exclude_self);
+    RVO_REQUIRE(path >= RVO_PATH_AUTO && path <= RVO_PATH_DENSE, "knn join: path %d (0 auto, 1 fp32 scan, 2 tcgen05, 3 dense fp32)",
+                (int)path);
+    const int k_max = exclude_self ? RVO_MAX_K - 1 : RVO_MAX_K;
+    RVO_REQUIRE(k >= 1 && k <= k_max, "knn join: k=%d outside 1..%d%s", k, k_max, exclude_self ? " (self mode)" : "");
+    RVO_REQUIRE(n_rows >= 0 && n_rows < (1ll << 31) && d > 0 && q_row_lo >= 0 && q_row_lo <= q_row_hi,
+                "knn join: bad shape n_rows=%lld query rows [%lld,%lld)", (long long)n_rows, (long long)q_row_lo,
+                (long long)q_row_hi);
+    RVO_REQUIRE(d_pad_in == (d + kBlockK - 1) / kBlockK * kBlockK, "knn join: d_pad must be d rounded up to 64");
+    RVO_REQUIRE(((uintptr_t)workspace & 1023) == 0 && ((uintptr_t)db & 15) == 0 && ((uintptr_t)qdb & 15) == 0 &&
+                    ((uintptr_t)q_rows & 7) == 0,
+                "knn join: alignment");
+    const long long nq = q_row_hi - q_row_lo;
+    RVO_REQUIRE((path != RVO_PATH_SMALL && path != RVO_PATH_DENSE) || (q_rows && nq <= RVO_SMALL_Q),
+                "knn join: the fp32 routes (path %d) take a q_rows list of at most %d rows, got %lld rows%s", (int)path, RVO_SMALL_Q,
+                nq, q_rows ? "" : " and no list");
+    if (qdb == db && !q_rows)
+        RVO_REQUIRE(q_row_hi <= n_rows, "knn join: query rows [%lld,%lld) outside the %lld rows of the DB", (long long)q_row_lo,
+                    (long long)q_row_hi, (long long)n_rows);
+    // both buffers on one device (the workspace's: search_impl takes the device from it)
+    int qdev = -1, tdev = -1, wdev = -1;
+    int rc = select_device_of(qdb, nullptr);
+    if (rc) return rc;
+    RVO_CUDA(cudaGetDevice(&qdev));
+    if (n_rows > 0) {
+        rc = select_device_of(db, nullptr);
+        if (rc) return rc;
+        RVO_CUDA(cudaGetDevice(&tdev));
+        RVO_REQUIRE(qdev == tdev, "knn join: query rows on device %d, target rows on device %d", qdev, tdev);
+    }
+    rc = select_device_of(workspace, nullptr);
+    if (rc) return rc;
+    RVO_CUDA(cudaGetDevice(&wdev));
+    RVO_REQUIRE(wdev == qdev, "knn join: workspace on device %d, query rows on device %d", wdev, qdev);
+    if (nq == 0) return RVO_OK;
+    KnnLayout L;
+    if (!knn_layout(n_rows, d, nq, k, path, &L)) {
+        set_error("knn join: no plan for n_rows=%lld d=%d k=%d path=%d", (long long)n_rows, d, k, (int)path);
+        return RVO_E_INVALID;
+    }
+    if (workspace_bytes < L.bytes) {
+        set_error("knn join workspace too small: %zu bytes given, %zu needed", workspace_bytes, L.bytes);
+        return RVO_E_WORKSPACE;
+    }
+    char* ws = (char*)workspace;
+    int64_t* lst_ids = (int64_t*)(ws + L.lists_off);
+    float* lst_scores = (float*)(ws + L.scores_off);
+    int32_t* lst_counts = (int32_t*)(ws + L.counts_off);
+    const int kk = exclude_self ? k + 1 : k;
+    for (long long i0 = q_row_lo; i0 < q_row_hi; i0 += L.block) {
+        const int nb = (int)(q_row_hi - i0 < L.block ? q_row_hi - i0 : L.block);
+        const StoredQueries sq{qdb, q_rows ? 0 : i0, q_rows ? q_rows + i0 : nullptr};
+        const size_t o = (size_t)(i0 - q_row_lo) * k;
+        rc = search_impl(db, n_rows, d, d_pad_in, nullptr, nb, kk, score_threshold, id_offset,
+                         exclude_self ? lst_ids : out_ids + o, exclude_self ? lst_scores : out_scores + o,
+                         exclude_self ? lst_counts : out_counts + (i0 - q_row_lo), workspace, L.search_bytes, stream, nullptr,
+                         L.search_path, &sq);
+        if (rc) return rc;
+        if (exclude_self) {
+            rc = launch_knn_exclude(lst_ids, lst_scores, lst_counts, nb, k, sq.row0, sq.rows, q_id_offset, out_ids + o,
+                                    out_scores + o, out_counts + (i0 - q_row_lo), stream);
+            if (rc) return rc;
+        }
+    }
+    return RVO_OK;
+}
+
+int rvo_knn_exclude_self(const int64_t* ids, const float* scores, const int32_t* counts, int32_t nq, int32_t k, int64_t q_row_lo,
+                         const int64_t* q_rows, int64_t q_id_offset, int64_t* out_ids, float* out_scores, int32_t* out_counts,
+                         void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(ids && scores && counts && out_ids && out_scores && out_counts, "knn exclude self: null pointer");
+    RVO_REQUIRE(nq >= 0 && k >= 1 && k < RVO_MAX_K, "knn exclude self: nq=%d k=%d (k outside 1..%d)", nq, k, RVO_MAX_K - 1);
+    RVO_REQUIRE((void*)ids != (void*)out_ids && (const void*)scores != (void*)out_scores, "knn exclude self: in place");
+    int rc = select_device_of(ids, nullptr);
+    if (rc) return rc;
+    return launch_knn_exclude(ids, scores, counts, nq, k, q_row_lo, q_rows, q_id_offset, out_ids, out_scores, out_counts,
+                              (cudaStream_t)stream);
 }
 
 // ---- peer-memory exchange (DESIGN.md §5) ------------------------------------------------------------------------------

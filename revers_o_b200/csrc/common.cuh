@@ -156,6 +156,9 @@ __host__ __device__ __forceinline__ size_t tiled_offset(long long row, int col, 
 // hence f >= t(k) - eps_q; so the k-th best f is >= t(k) - eps_q, and every row of the true top-k has tensor score
 // >= t(k) - 2 eps_q.  Thresholds taken from tensor-core scores are therefore lowered by margin = 2 eps_q, where eps_q
 // also carries 2^-13 of slack for fp32 accumulation-order differences between tile shapes and the fp32 FMA re-score.
+// A STORED row as the query (rvo_knn_join) is its own bf16 operand: bf16(q) == q, so ||bf16(q) - q|| = 0 and eps_q is the
+// accumulation slack alone, query_margin(0) = 2^-12.  The re-score query is the exact fp32 upconvert of the same row, so the
+// bound above holds unchanged with the raw (not re-normalised) row; ||q|| <= 1 + 2^-8 like any stored row.
 __host__ __device__ __forceinline__ float query_margin(float bf16_err_norm) {
     return 2.0f * (bf16_err_norm * (1.0f + 0.00390625f) + 0.0001220703125f);
 }

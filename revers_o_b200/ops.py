@@ -485,6 +485,105 @@ def components_exact(db: torch.Tensor, n_rows: int, d: int, threshold: float, id
         return labels + int(id_offset), m
 
 
+def knn_join(qdb: torch.Tensor, q_row_lo: int, q_row_hi: int, q_id_offset: int, db: torch.Tensor, n_rows: int, d: int, k: int,
+             score_threshold: float | None, id_offset: int, exclude_self: bool, q_rows: torch.Tensor | None = None, path: int = 0,
+             out=None):
+    """rvo_knn_join: for each query row of the tiled storage `qdb` — rows [q_row_lo, q_row_hi), or q_rows[q_row_lo:q_row_hi]
+    when a device int64 list is given — the k rows of the first n_rows rows of `db` with the highest fp32 dot of the two stored
+    rows.  `exclude_self` (qdb and db one collection, ids row + offset): a row's own id is left out of its list.  Returns device
+    tensors (ids int64 [nq, k], scores f32 [nq, k], counts int32 [nq]) as `search_topk` does; counts[q] == -1 marks a query that
+    overflowed the fused path (`knn_exact`).  Async on the current stream of db's device."""
+    require_cuda(qdb, "qdb")
+    require_cuda(db, "db")
+    for t in (qdb, db):
+        assert t.dtype == torch.bfloat16 and t.dim() == 4 and t.is_contiguous() and t.shape[1] * TILE_COLS == d_pad_of(d)
+    assert n_rows <= db_capacity(db) and qdb.device == db.device
+    if q_rows is None:
+        assert q_row_hi <= db_capacity(qdb)
+    else:
+        assert q_rows.dtype == torch.int64 and q_rows.is_contiguous() and q_rows.device == db.device and q_row_hi <= q_rows.numel()
+    k_max = RVO_MAX_K - 1 if exclude_self else RVO_MAX_K
+    if not 1 <= k <= k_max:
+        raise RvoError(f"k={k} outside 1..{k_max}" + (" (a row's own match is left out)" if exclude_self else ""))
+    nq = int(q_row_hi) - int(q_row_lo)
+    dev = db.device
+    if out is None:
+        out = (torch.empty((nq, k), dtype=torch.int64, device=dev), torch.empty((nq, k), dtype=torch.float32, device=dev),
+               torch.empty((nq,), dtype=torch.int32, device=dev))
+    ids, scores, counts = out
+    if nq == 0:
+        return ids, scores, counts
+    lib = _lib.load()
+    nbytes = lib.rvo_knn_workspace_bytes(int(n_rows), d, nq, k, int(path))
+    if nbytes == 0:
+        raise RvoError(f"rvo_knn_workspace_bytes rejected n_rows={n_rows} d={d} nq={nq} k={k} path={path}")
+    ws = workspace(dev, nbytes, "knn")
+    thr = -math.inf if score_threshold is None else float(score_threshold)
+    check(lib.rvo_knn_join(_ptr(qdb), int(q_row_lo), int(q_row_hi), _ptr(q_rows), int(q_id_offset), _ptr(db), int(n_rows), d,
+                           d_pad_of(d), int(k), thr, int(id_offset), int(bool(exclude_self)), int(path), _ptr(ids), _ptr(scores),
+                           _ptr(counts), _ptr(ws), nbytes, _stream(dev)), "rvo_knn_join")
+    return ids, scores, counts
+
+
+def knn_exact(qdb: torch.Tensor, q_row_lo: int, q_row_hi: int, q_id_offset: int, db: torch.Tensor, n_rows: int, d: int, k: int,
+              score_threshold: float | None, id_offset: int, exclude_self: bool, q_rows: torch.Tensor | None = None):
+    """`knn_join` plus the overflow protocol of `search_topk_exact`: rows the fused path flags -1 are re-run, as a q_rows list, in
+    batches of <= RVO_SMALL_Q through the exact fp32 scan, and what that route flags as well through the dense fp32 route, which
+    cannot overflow.  Scores stay the raw dot of the stored rows on every route.  Rows wider than 2048 (d_pad) have no fp32
+    route, as in `search_topk_exact`: a flagged row stays -1 there (the public layer raises).  Synchronises (reads counts)."""
+    ids, scores, counts = knn_join(qdb, q_row_lo, q_row_hi, q_id_offset, db, n_rows, d, k, score_threshold, id_offset, exclude_self,
+                                   q_rows)
+    bad = (counts < 0).nonzero().flatten()                      # host sync; pathological inputs only take the branch
+    if bad.numel() == 0 or d_pad_of(d) > 2048:
+        return ids, scores, counts
+    rows = bad + int(q_row_lo) if q_rows is None else q_rows[int(q_row_lo):int(q_row_hi)][bad]
+    a, b, c = knn_fp32(qdb, rows, q_id_offset, db, n_rows, d, k, score_threshold, id_offset, exclude_self)
+    ids[bad], scores[bad], counts[bad] = a, b, c
+    return ids, scores, counts
+
+
+def knn_fp32(qdb: torch.Tensor, q_rows: torch.Tensor, q_id_offset: int, db: torch.Tensor, n_rows: int, d: int, k: int,
+             score_threshold: float | None, id_offset: int, exclude_self: bool):
+    """The exact routes of `knn_exact` for the query rows listed in q_rows (device int64): batches of <= RVO_SMALL_Q through the
+    fp32 scan, then what that route flags through the dense fp32 route, which cannot overflow.  Every pair is scored by the
+    same fp32 arithmetic on both routes, whichever rows the target holds.  Needs d_pad <= 2048.  Returns device tensors as
+    `knn_join`; synchronises."""
+    nq = q_rows.numel()
+    dev = db.device
+    ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
+    counts = torch.full((nq,), -1, dtype=torch.int32, device=dev)
+    todo = list(range(nq))
+    for path in (_lib.RVO_PATH_SMALL, _lib.RVO_PATH_DENSE):
+        for i in range(0, len(todo), RVO_SMALL_Q):
+            sel = torch.tensor(todo[i:i + RVO_SMALL_Q], device=dev)
+            a, b, c = knn_join(qdb, 0, sel.numel(), q_id_offset, db, n_rows, d, k, score_threshold, id_offset, exclude_self,
+                               q_rows[sel], path)
+            ids[sel], scores[sel], counts[sel] = a, b, c
+        todo = (counts < 0).nonzero().flatten().tolist()
+        if not todo:
+            break
+    return ids, scores, counts
+
+
+def knn_exclude_self(ids: torch.Tensor, scores: torch.Tensor, counts: torch.Tensor, q_row_lo: int, q_id_offset: int,
+                     q_rows: torch.Tensor | None = None):
+    """rvo_knn_exclude_self: lists of k + 1 (ids [nq, k+1], scores, counts [nq]) -> lists of k without each query's own id,
+    q_id_offset + (q_rows[q] if a list is given else q_row_lo + q).  Async."""
+    require_cuda(ids, "ids")
+    nq, k1 = ids.shape
+    assert ids.is_contiguous() and scores.is_contiguous() and counts.is_contiguous() and scores.shape == ids.shape
+    if q_rows is not None:
+        assert q_rows.dtype == torch.int64 and q_rows.is_contiguous() and q_rows.numel() >= nq and q_rows.device == ids.device
+    dev = ids.device
+    oi = torch.empty((nq, k1 - 1), dtype=torch.int64, device=dev)
+    os_ = torch.empty((nq, k1 - 1), dtype=torch.float32, device=dev)
+    oc = torch.empty((nq,), dtype=torch.int32, device=dev)
+    check(_lib.load().rvo_knn_exclude_self(_ptr(ids), _ptr(scores), _ptr(counts), nq, k1 - 1, int(q_row_lo), _ptr(q_rows),
+                                           int(q_id_offset), _ptr(oi), _ptr(os_), _ptr(oc), _stream(dev)), "rvo_knn_exclude_self")
+    return oi, os_, oc
+
+
 def merge_topk(ids: torch.Tensor, scores: torch.Tensor, counts: torch.Tensor, k: int):
     """K3.  ids int64 [G,nq,k], scores f32 [G,nq,k], counts int32 [G,nq] -> merged (ids, scores, counts)."""
     require_cuda(ids, "ids")

@@ -13,7 +13,9 @@ The self-join of a collection row-sharded over the devices of ONE process (B200V
 here too: `selfjoin_plan` (pure host logic) and `selfjoin_sharded`, which joins the shards where they live and moves only
 query blocks.  So is the join between two such collections (B200VectorDB.join_collections): `crossjoin_plan` and
 `crossjoin_sharded`, run by the same device loop, and the duplicate groups of a row-sharded collection
-(B200VectorDB.find_duplicate_groups): `components_sharded`, the self-join's items unioned into one forest per device.
+(B200VectorDB.find_duplicate_groups): `components_sharded`, the self-join's items unioned into one forest per device.  The
+k-nearest-neighbour join of two such collections, or of one with itself (B200VectorDB.knn_join), is `knn_plan` and `knn_sharded`:
+per-shard lists merged by K3 on the left shard's device, sharing the staging code (`_Staging`) of the joins.
 """
 from __future__ import annotations
 
@@ -307,6 +309,181 @@ def _join_on_devices(shards: list, items: dict, d: int, threshold: float, max_pa
     return np.concatenate([done[dv][0] for dv in sorted(done)]), np.concatenate([done[dv][1] for dv in sorted(done)])
 
 
+class KnnItem(NamedTuple):
+    """Query rows [q_lo, q_hi) of left shard q_shard against every row of right shard t_shard, on the right shard's device."""
+    q_shard: int
+    q_lo: int
+    q_hi: int
+    t_shard: int
+
+
+def knn_plan(left: list, right: list, block: int = 8192) -> dict[int, list[KnnItem]]:
+    """Work of the kNN join of two row-sharded collections: left and right are [(device index, rows)].  Returns {device index of
+    a right shard: items that run there}.  Every left shard is cut into query blocks of `block` rows (a multiple of 128, so a
+    block is whole tiles), and every (query block, right shard) pair is one item on the right shard's device: right shards never
+    move, query blocks do.  Each device's items come block by block in left row order."""
+    if block <= 0 or block % ops.TILE_ROWS:
+        raise _lib.RvoError(f"kNN join query blocks must be a positive multiple of {ops.TILE_ROWS} rows, got {block}")
+    plan: dict[int, list[KnnItem]] = {int(dv): [] for dv, _ in right}
+    for a, (_, na) in enumerate(left):
+        for lo in range(0, int(na), block):
+            for b, (dv, nb) in enumerate(right):
+                if int(nb):
+                    plan[int(dv)].append(KnnItem(a, lo, min(lo + block, int(na)), b))
+    return plan
+
+
+def knn_sharded(left: list, right: list, d: int, k: int, score_threshold: float | None, exclude_self: bool,
+                device_ms: dict | None = None, block: int = 8192, chunk: int = 1 << 18):
+    """kNN join of two collections, each row-sharded over devices of one process: for every left row, in row order, the k
+    right rows with the highest fp32 dot of the two stored rows.  left, right: [(tiled storage, rows, first global row)], the
+    left shards in row order; `exclude_self` (left and right are one collection): a row's own match is left out.  Returns host
+    arrays (rows int64 [N_L, k] of global right rows, -1 pad; scores f32 [N_L, k], -inf pad; counts int32 [N_L]); a count of -1
+    remains only for rows wider than 2048 that overflowed (`ops.knn_exact`).  Equal to the single-device result: ids identical,
+    scores equal up to the last bits where one layout took the fp32 route for a row and the other did not.
+
+    Results go to pinned host memory as they are made, so device memory does not grow with the left collection.  One shard
+    on one device: one `rvo_knn_join` call per `chunk` left rows into one reusable device buffer (12 * chunk * k bytes).
+    Otherwise `knn_plan`'s items run with k' = k + 1 (self mode) or k lists each, one query block (`block` rows, a multiple of
+    128) at a time, enqueued before any synchronisation: for each block, every right shard's device joins it (a block of another
+    device is peer-copied into that device's staging blocks, `_Staging`) into that shard's reusable list buffer [block, k']; the
+    lists are peer-copied into the block's home device's gather buffer [shards, block, k'], merged there (`rvo_merge_topk`: at
+    most 64 right shards, shards * k' <= 4096), stripped of the row itself (self mode) and copied to pinned host memory.
+    Per device that is 12 * block * k' bytes per right shard it holds, 12 * shards * block * k' bytes of gather buffer if it
+    holds left rows, two staging blocks and one search workspace.  A cross-device copy orders both devices' current streams
+    around it, so a buffer is rewritten only after its previous contents have been copied or merged.  Rows the merge flags -1
+    are then re-run through the exact fp32 routes (`ops.knn_fp32`) on every right shard and merged again, as the sharded search
+    does.  `device_ms`: each device's busy time (CUDA events, ms) of the enqueued work."""
+    if block <= 0 or block % ops.TILE_ROWS:
+        raise _lib.RvoError(f"kNN join query blocks must be a positive multiple of {ops.TILE_ROWS} rows, got {block}")
+    kk = k + 1 if exclude_self else k
+    G = len(right)
+    n_left = sum(int(n) for _, n, _ in left)
+    out_i = torch.full((n_left, k), -1, dtype=torch.int64).pin_memory()
+    out_s = torch.full((n_left, k), -float("inf"), dtype=torch.float32).pin_memory()
+    out_c = torch.zeros((n_left,), dtype=torch.int32).pin_memory()
+    if n_left == 0 or G == 0:
+        return out_i.numpy(), out_s.numpy(), out_c.numpy()
+    single = len(left) == 1 and G == 1 and left[0][0].device == right[0][0].device
+    if not single and (G > 64 or G * kk > 4096):
+        raise _lib.RvoError(f"kNN join over {G} right shards with {kk} candidates each: the merge takes at most 64 shards and "
+                            "4096 candidates per row")
+    offs = [0]
+    for _, n, _ in left:
+        offs.append(offs[-1] + int(n))
+    ready = {}                     # copies read a shard after what its device's current stream had queued before the join
+    for v, _, _ in list(left) + list(right):
+        if v.device.index not in ready:
+            ready[v.device.index] = torch.cuda.Event()
+            ready[v.device.index].record(torch.cuda.current_stream(v.device))
+    st = {dv: _Staging(torch.device("cuda", dv), d, block, ready) for dv in ready}
+    if single:
+        (qv, nl, q0), (tv, nr, t0) = left[0], right[0]
+        m = min(chunk, nl)
+        buf = (torch.empty((m, k), dtype=torch.int64, device=tv.device), torch.empty((m, k), dtype=torch.float32, device=tv.device),
+               torch.empty((m,), dtype=torch.int32, device=tv.device))
+        with torch.cuda.device(tv.device):
+            for lo in range(0, nl, m):
+                hi = min(nl, lo + m)
+                res = ops.knn_join(qv, lo, hi, q0, tv, nr, d, k, score_threshold, t0, exclude_self,
+                                   out=tuple(x[: hi - lo] for x in buf))
+                for dst, src in zip((out_i, out_s, out_c), res):      # stream-ordered before the next call rewrites buf
+                    dst[lo:hi].copy_(src, non_blocking=True)
+    else:
+        _knn_blocks(left, right, offs, d, k, kk, score_threshold, exclude_self, block, st, (out_i, out_s, out_c))
+    for s in st.values():
+        s.stop.record(torch.cuda.current_stream(s.dev))
+    for dv in sorted(st):
+        torch.cuda.current_stream(torch.device("cuda", dv)).synchronize()
+    if device_ms is not None:
+        for dv, s in st.items():
+            device_ms[dv] = s.start.elapsed_time(s.stop)
+    for a, (qv, nl, q0) in enumerate(left):
+        bad = (out_c[offs[a]: offs[a] + int(nl)] < 0).nonzero().flatten()
+        if bad.numel():
+            _knn_overflow(left[a], offs[a], bad, right, d, k, kk, score_threshold, exclude_self, (out_i, out_s, out_c))
+    return out_i.numpy(), out_s.numpy(), out_c.numpy()
+
+
+def _knn_blocks(left: list, right: list, offs: list, d: int, k: int, kk: int, score_threshold, exclude_self: bool, block: int,
+                st: dict, out: tuple) -> None:
+    """The block pipeline of `knn_sharded` (several shards): enqueues, for every query block of `knn_plan` in left row order,
+    the joins on the right shards' devices, the peer copies of their lists to the block's home device, the merge, the exclusion
+    and the copy into the pinned host outputs `out`.  Nothing synchronises."""
+    G = len(right)
+    parts = [(torch.empty((block, kk), dtype=torch.int64, device=tv.device),
+              torch.empty((block, kk), dtype=torch.float32, device=tv.device),
+              torch.empty((block,), dtype=torch.int32, device=tv.device)) for tv, _, _ in right]
+    gather = {}
+    for qv, nl, _ in left:
+        if nl and qv.device.index not in gather:
+            dev = qv.device
+            gather[dev.index] = (torch.empty(G * block * kk, dtype=torch.int64, device=dev),
+                                 torch.empty(G * block * kk, dtype=torch.float32, device=dev),
+                                 torch.empty(G * block, dtype=torch.int32, device=dev))
+    plan = knn_plan([(v.device.index, n) for v, n, _ in left], [(v.device.index, n) for v, n, _ in right], block)
+    blocks: dict = {}                                  # (left shard, q_lo) -> (q_hi, [items]) in left row order
+    for dv, its in plan.items():
+        for it in its:
+            blocks.setdefault((it.q_shard, it.q_lo), (it.q_hi, []))[1].append(it)
+    for (a, lo), (hi, its) in sorted(blocks.items()):
+        qv, _, q0 = left[a]
+        nb = hi - lo
+        for it in its:
+            tv, nr, t0 = right[it.t_shard]
+            s = st[tv.device.index]
+            qdb, q_lo, q_hi, q_off, slot = s.stage(qv, lo, hi, q0)
+            pi, ps, pc = parts[it.t_shard]
+            with torch.cuda.device(s.dev):
+                ops.knn_join(qdb, q_lo, q_hi, q_off, tv, nr, d, kk, score_threshold, t0, False, out=(pi[:nb], ps[:nb], pc[:nb]))
+            s.release(slot)
+        home = qv.device
+        fi, fs, fc = gather[home.index]
+        gi, gs, gc = fi[: G * nb * kk].view(G, nb, kk), fs[: G * nb * kk].view(G, nb, kk), fc[: G * nb].view(G, nb)
+        with torch.cuda.device(home):
+            for it in its:                             # peer copies: after the join on its device, before the merge here
+                pi, ps, pc = parts[it.t_shard]
+                gi[it.t_shard].copy_(pi[:nb], non_blocking=True)
+                gs[it.t_shard].copy_(ps[:nb], non_blocking=True)
+                gc[it.t_shard].copy_(pc[:nb], non_blocking=True)
+            res = ops.merge_topk(gi, gs, gc, kk)
+            if exclude_self:
+                res = ops.knn_exclude_self(*res, lo, q0)
+            o0 = offs[a] + lo
+            for dst, src in zip(out, res):
+                dst[o0:o0 + nb].copy_(src, non_blocking=True)
+
+
+def _knn_overflow(left_shard, off: int, bad: torch.Tensor, right: list, d: int, k: int, kk: int, score_threshold,
+                  exclude_self: bool, out: tuple) -> None:
+    """Overflow protocol of `knn_sharded` for the flagged local rows `bad` of one left shard: their tiles are copied to every
+    right shard's device, the exact fp32 routes (`ops.knn_fp32`) run them there as a q_rows list, and the lists are merged on
+    the left shard's device (then the row itself is left out) into rows off + bad of the host outputs.  Every shard scores such
+    a row with the same fp32 arithmetic, as the single-device protocol does over all the rows.  Rows wider than 2048 have no
+    fp32 route and stay flagged.  Synchronises."""
+    qv, _, q0 = left_shard
+    if ops.d_pad_of(d) > 2048:
+        return
+    home = qv.device
+    rows = bad.to(home)
+    tiles, slot = torch.unique(rows // ops.TILE_ROWS, return_inverse=True)
+    stage = qv[tiles]                                          # the tiles holding the flagged rows
+    local = slot * ops.TILE_ROWS + rows % ops.TILE_ROWS        # their rows inside the staged tiles
+    parts = []
+    for tv, nr, t0 in right:
+        with torch.cuda.device(tv.device):
+            qd, qr = stage.to(tv.device), local.to(tv.device)
+            parts.append(ops.knn_fp32(qd, qr, 0, tv, nr, d, kk, score_threshold, t0, False))
+    with torch.cuda.device(home):
+        res = ops.merge_topk(torch.stack([p[0].to(home) for p in parts]), torch.stack([p[1].to(home) for p in parts]),
+                             torch.stack([p[2].to(home) for p in parts]), kk)
+        if exclude_self:
+            res = ops.knn_exclude_self(*res, 0, q0, rows)
+        idx = bad + off
+        for dst, src in zip(out, res):
+            dst[idx] = src.cpu()
+
+
 def _join_runs(its: list[JoinItem], shards: list, dv: int) -> list[JoinItem]:
     """The items of one device as calls: consecutive items that read their query rows in place (same device) and share a
     target merge into one call (the C entry walks the query blocks itself); a query block of another device stays one call."""
@@ -323,17 +500,12 @@ def _join_runs(its: list[JoinItem], shards: list, dv: int) -> list[JoinItem]:
     return runs
 
 
-class _JoinState:
-    """Output (a pair buffer, or a union-find forest), staging blocks and streams of one device during `_join_on_devices`."""
+class _Staging:
+    """Staging blocks, copy streams and busy-time events of one device: query blocks of shards on other devices are peer-copied
+    into one of two staging blocks here, so the copy of one block overlaps the work on the other (`_JoinState`, `knn_sharded`)."""
 
-    def __init__(self, dev: torch.device, out_cap: int, d: int, block: int, ready: dict, n_left: int | None = None,
-                 parent: torch.Tensor | None = None):
-        self.dev, self.ready, self.n_left = dev, ready, n_left
-        if parent is None:
-            self.out, self.join = ops.join_out(out_cap, dev), ops.join_threshold
-        else:       # the forest of earlier attempts is kept; the hit count and overflow counter start at 0
-            self.out = (parent, torch.zeros((1,), dtype=torch.int64, device=dev), torch.zeros((1,), dtype=torch.int32, device=dev))
-            self.join = ops.join_components
+    def __init__(self, dev: torch.device, d: int, block: int, ready: dict):
+        self.dev, self.ready = dev, ready
         self.d, self.block = d, block
         self.slots: list = []                    # two staging blocks: the copy of one overlaps the join of the other
         self.free: list = []                     # event per slot: the join that last read it has finished
@@ -343,46 +515,68 @@ class _JoinState:
         self.start, self.stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         self.start.record(torch.cuda.current_stream(dev))
 
+    def stage(self, qv: torch.Tensor, q_lo: int, q_hi: int, q_row0: int):
+        """Query rows [q_lo, q_hi) (at most `block`) of the tiled storage qv, whose first global row is q_row0, as seen from this
+        device: (tiled storage, lo, hi, first global row of that storage, staging slot or None).  Rows of this device are read
+        in place; others are copied, ordered after the source device's current stream as it was when `ready` was recorded and
+        before this device's current stream.  Pass the slot to `release` after the work that reads it is enqueued."""
+        if qv.device == self.dev:
+            return qv, q_lo, q_hi, q_row0, None
+        b0, b1 = q_lo // ops.TILE_ROWS, (q_hi + ops.TILE_ROWS - 1) // ops.TILE_ROWS
+        if not self.slots:
+            self.slots = [ops.db_alloc(self.block, self.d, self.dev) for _ in range(2)]
+            self.free = [None, None]
+            self.copy_stream = torch.cuda.Stream(self.dev)
+        k = self.next % 2
+        self.next += 1
+        src = self.src_streams.get(qv.device.index)
+        if src is None:
+            src = self.src_streams[qv.device.index] = torch.cuda.Stream(qv.device)
+            src.wait_event(self.ready[qv.device.index])
+        if self.free[k] is not None:
+            self.copy_stream.wait_event(self.free[k])
+        # a cross-device copy_ runs on the source device's current stream, after the destination device's current stream
+        with torch.cuda.stream(src), torch.cuda.stream(self.copy_stream):
+            self.slots[k][: b1 - b0].copy_(qv[b0:b1], non_blocking=True)
+        torch.cuda.current_stream(self.dev).wait_stream(self.copy_stream)
+        return self.slots[k], q_lo - b0 * ops.TILE_ROWS, q_hi - b0 * ops.TILE_ROWS, q_row0 + b0 * ops.TILE_ROWS, k
+
+    def release(self, slot) -> None:
+        if slot is not None:
+            ev = torch.cuda.Event()
+            ev.record(torch.cuda.current_stream(self.dev))
+            self.free[slot] = ev
+
+
+class _JoinState(_Staging):
+    """Output (a pair buffer, or a union-find forest), staging blocks and streams of one device during `_join_on_devices`."""
+
+    def __init__(self, dev: torch.device, out_cap: int, d: int, block: int, ready: dict, n_left: int | None = None,
+                 parent: torch.Tensor | None = None):
+        super().__init__(dev, d, block, ready)
+        self.n_left = n_left
+        if parent is None:
+            self.out, self.join = ops.join_out(out_cap, dev), ops.join_threshold
+        else:       # the forest of earlier attempts is kept; the hit count and overflow counter start at 0
+            self.out = (parent, torch.zeros((1,), dtype=torch.int64, device=dev), torch.zeros((1,), dtype=torch.int32, device=dev))
+            self.join = ops.join_components
+
     def run(self, it: JoinItem, shards: list, d: int, threshold: float, cand_cap: int) -> None:
         qv, _, q_row0 = shards[it.q_shard]
         tv, _, t_row0 = shards[it.t_shard]
-        cur = torch.cuda.current_stream(self.dev)
         if it.q_shard == it.t_shard:
             with torch.cuda.device(self.dev):
                 self.join(tv, it.q_lo, it.q_hi, t_row0, tv, it.t_hi, d, threshold, t_row0, cand_cap, self.out)
             return
         target = tv[it.t_lo // ops.TILE_ROWS:]
-        if qv.device == self.dev:
-            qdb, q_lo, q_hi, q_off = qv, it.q_lo, it.q_hi, q_row0
-        else:
-            b0, b1 = it.q_lo // ops.TILE_ROWS, (it.q_hi + ops.TILE_ROWS - 1) // ops.TILE_ROWS
-            if not self.slots:
-                self.slots = [ops.db_alloc(self.block, d, self.dev) for _ in range(2)]
-                self.free = [None, None]
-                self.copy_stream = torch.cuda.Stream(self.dev)
-            k = self.next % 2
-            self.next += 1
-            src = self.src_streams.get(qv.device.index)
-            if src is None:
-                src = self.src_streams[qv.device.index] = torch.cuda.Stream(qv.device)
-                src.wait_event(self.ready[qv.device.index])
-            if self.free[k] is not None:
-                self.copy_stream.wait_event(self.free[k])
-            # a cross-device copy_ runs on the source device's current stream, after the destination device's current stream
-            with torch.cuda.stream(src), torch.cuda.stream(self.copy_stream):
-                self.slots[k][: b1 - b0].copy_(qv[b0:b1], non_blocking=True)
-            cur.wait_stream(self.copy_stream)
-            qdb, q_lo, q_hi, q_off = self.slots[k], it.q_lo - b0 * ops.TILE_ROWS, it.q_hi - b0 * ops.TILE_ROWS, q_row0 + b0 * ops.TILE_ROWS
+        qdb, q_lo, q_hi, q_off, slot = self.stage(qv, it.q_lo, it.q_hi, q_row0)
         with torch.cuda.device(self.dev):
             if self.n_left is None:
                 self.join(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo, cand_cap, self.out)
             else:
                 ops.cross_join_threshold(qdb, q_lo, q_hi, q_off, target, it.t_hi - it.t_lo, d, threshold, t_row0 + it.t_lo,
                                          it.q_shard >= self.n_left, cand_cap, self.out)
-        if qdb is not qv:
-            ev = torch.cuda.Event()
-            ev.record(cur)
-            self.free[k] = ev
+        self.release(slot)
 
 
 class ShardedIndex:

@@ -774,6 +774,45 @@ class B200VectorDB:
         p, sc = crossjoin_sharded(left, right, a.dim, threshold, max_pairs=max_pairs)
         return a, b, p, sc
 
+    def knn_join(self, collection_name: str, k: int = 10, score_threshold: float | None = None,
+                 other_collection_name: str | None = None, other: B200VectorDB | None = None):
+        """The k best matches of every stored point: for each row of `collection_name`, in row order, the k rows of the other
+        collection with the highest score, the fp32 dot of the two stored rows (the score `find_near_duplicates` and
+        `join_collections` report for the same pair).  With no other collection the collection is matched against itself and a
+        row's own match is left out (its exact copies are kept, in row order); k <= 511 then, k <= 512 across two collections.
+        `other` is the B200VectorDB holding the other collection (by default this one).  Hits below `score_threshold` are
+        dropped (equal is kept).  Returns numpy (rows int64 [n, k] of rows of the other collection, -1 padded; scores float32
+        [n, k], -inf padded; counts int32 [n]), ordered like `search_batch`'s output (score descending, ties by lower row): map
+        rows to ids and payloads as for `search_batch`.  Exact on any data, row-sharded collections included
+        (`sharded.knn_sharded`).  Both databases stay read-locked for the call."""
+        other = self if other is None else other
+        with self._read_both(other):
+            return self._knn_rows(collection_name, k, score_threshold, other_collection_name, other)
+
+    def _knn_rows(self, collection_name: str, k: int, score_threshold: float | None, other_collection_name: str | None,
+                  other: B200VectorDB):
+        """`knn_join`; the caller holds both read locks."""
+        from .sharded import knn_sharded
+        exclude = other_collection_name is None
+        if exclude and other is not self:
+            raise RvoError("knn_join: name the other database's collection (other_collection_name)")
+        a = self._coll(collection_name)
+        b = a if exclude else other._coll(other_collection_name)
+        if b.dim != a.dim:
+            raise RvoError(f"Wrong input: Vector dimension error: expected dim: {a.dim}, got {b.dim}")
+        k = int(k)
+        k_max = RVO_MAX_K - 1 if exclude else RVO_MAX_K
+        if not 1 <= k <= k_max:
+            raise RvoError(f"knn_join: k={k} outside 1..{k_max}" + (" (a point's own match is left out)" if exclude else ""))
+        left = [(s.vectors, s.n, s.row0) for s in a.shards if s.n]
+        right = [(s.vectors, s.n, s.row0) for s in b.shards if s.n]
+        rows, scores, counts = knn_sharded(left, right, a.dim, k, score_threshold, exclude)
+        bad = np.flatnonzero(counts < 0)
+        if bad.size:
+            raise RvoError(f"knn_join: rows {bad[:20].tolist()}{' ...' if bad.size > 20 else ''} overflowed the candidate lists "
+                           f"and rows of {a.dim} dims (> 2048) have no exact fp32 route")
+        return rows, scores, counts
+
     def count(self, collection_name: str) -> int:
         return self._coll(collection_name).n
 
@@ -1057,6 +1096,28 @@ def group_labels(labels, min_size: int = 2, row0: int = 0) -> list:
     keep = np.flatnonzero(sizes >= max(int(min_size), 1))
     keep = keep[np.lexsort((order[starts[keep]], -sizes[keep]))]
     return [(order[starts[k]: starts[k] + sizes[k]] + row0).tolist() for k in keep]
+
+
+def mutual_best(rows_ab, counts_ab, rows_ba, counts_ba, scores_ab):
+    """One-to-one correspondences between two collections A and B from their kNN lists (`B200VectorDB.knn_join`, A -> B and
+    B -> A; only each list's first entry is read): the pairs (a, b) where b is a's best match and a is b's best match.
+    `scores_ab` (the A -> B scores, [n_A, k]) gives each pair its score: the lists B -> A carry the same pair's score as well,
+    but the order and the returned scores are defined on the side whose first entries name the pairs.
+    Returns (pairs int64 [m, 2] of (a row, b row), scores float32 [m]), score descending, ties by a, then b."""
+    rows_ab, rows_ba = np.asarray(rows_ab, dtype=np.int64), np.asarray(rows_ba, dtype=np.int64)
+    counts_ab, counts_ba = np.asarray(counts_ab), np.asarray(counts_ba)
+    scores_ab = np.asarray(scores_ab, dtype=np.float32)
+    a = np.flatnonzero(counts_ab > 0)
+    b = rows_ab[a, 0] if a.size else np.zeros(0, np.int64)
+    keep = np.zeros(a.size, bool)
+    if a.size and len(counts_ba):
+        ok = (b >= 0) & (b < len(counts_ba))
+        bo = b[ok]
+        keep[ok] = (counts_ba[bo] > 0) & (rows_ba[bo, 0] == a[ok])
+    a, b = a[keep], b[keep]
+    s = scores_ab[a, 0] if a.size else np.zeros(0, np.float32)
+    o = np.lexsort((b, a, -s.astype(np.float64)))
+    return np.stack([a[o], b[o]], 1).astype(np.int64).reshape(-1, 2), s[o].astype(np.float32)
 
 
 def _copy_blocks_to_device(view: np.ndarray, dst: torch.Tensor, chunk_blocks: int = 4096) -> None:
