@@ -375,6 +375,34 @@ int rvo_knn_exclude_self(const int64_t* ids, const float* scores, const int32_t*
                          int32_t* out_counts, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Spherical k-means (B200VectorDB.cluster).  Centroids are stored like rows (L2-normalised bf16, tiled, cluster c = row c);
+ * a row's label is its rvo_knn_join(k = 1) match against the centroid buffer (ties by the lower index).  The update step:
+ * rvo_kmeans_update reads the assignment of rows [row_lo, row_hi) of the tiled storage `db`:
+ *   ids        [dev] int64 [n] (n = row_hi - row_lo; the k = 1 lists): cluster = ids[i] - id_offset, -1 outside [0, n_clusters)
+ *   prev_labels  [dev] int32 [n] or NULL: the previous labels (NULL: every row counts as changed)
+ *   labels     [dev] int32 [n] out: the clusters, -1 for ids outside the range (such rows add nothing)
+ *   sums       [dev] int64 [n_clusters][d], ADDED to: each member's bf16 components as integers rint(x * 2^31) (exact for
+ *              |x| >= 2^-24; below 2^63 for fewer than 2^31 rows).  Integer addition, so the sums are bit-identical whatever the
+ *              launch configuration, the block order or the split of the rows into calls (shards).
+ *   counts     [dev] int64 [n_clusters], ADDED to: members per cluster
+ *   changed    [dev] int64 [1], ADDED to: rows whose label differs from prev_labels
+ *   workspace  [dev] rvo_kmeans_update_workspace_bytes(n, n_clusters) bytes, 256-B aligned
+ * db and sums on one device; 1 <= n_clusters <= RVO_KMEANS_MAX_CLUSTERS, n < 2^31.
+ * rvo_kmeans_finalize: the new centroids from the (reduced) sums: scratch_f32 [n_clusters][d] = sums * 2^-31 in fp32, then the
+ * rows normalised and rounded into the tiled centroid storage `centroids` exactly as rvo_normalize_rows does (an all-zero row
+ * stays zero).  out_empty [n_clusters] int32 = 1 for a cluster with no member or an all-zero sum (re-seeded by the caller),
+ * n_empty [dev] int64 [1] is ADDED to by their number.
+ * All are asynchronous on `stream`.
+ * ---------------------------------------------------------------------------------------------- */
+#define RVO_KMEANS_MAX_CLUSTERS 65536
+size_t rvo_kmeans_update_workspace_bytes(int64_t n_rows, int32_t n_clusters);
+int rvo_kmeans_update(const uint16_t* db, int64_t row_lo, int64_t row_hi, int32_t d, int64_t d_pad, const int64_t* ids,
+                      int64_t id_offset, int32_t n_clusters, const int32_t* prev_labels, int32_t* labels, int64_t* sums,
+                      int64_t* counts, int64_t* changed, void* workspace, size_t workspace_bytes, void* stream);
+int rvo_kmeans_finalize(const int64_t* sums, const int64_t* counts, int32_t n_clusters, int32_t d, float* scratch_f32,
+                        uint16_t* centroids, int32_t* out_empty, int64_t* n_empty, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Counters for bench.py's `gpu_launches` claim: number of kernels THIS library has launched on the
  * calling process since load (monotonic).
  * ---------------------------------------------------------------------------------------------- */

@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("RVO_LIB_PATH") or os.path.join(_HERE, "lib", "libreve
 RVO_E_UNSUPPORTED = -5
 RVO_MAX_K = 512
 RVO_SMALL_Q = 4
+RVO_KMEANS_MAX_CLUSTERS = 65536
 RVO_DTYPE_BF16, RVO_DTYPE_F16 = 0, 1
 RVO_PATH_AUTO, RVO_PATH_SMALL, RVO_PATH_TENSOR, RVO_PATH_DENSE = 0, 1, 2, 3
 
@@ -88,6 +89,11 @@ PROTOTYPES = {
                                C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "rvo_knn_exclude_self": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_void_p,
                                        C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rvo_kmeans_update_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
+    "rvo_kmeans_update": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_int64, C.c_int32,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rvo_kmeans_finalize": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p]),
     "rvo_kernel_launch_count": (C.c_int64, []),
     "rvo_last_scan_ms": (C.c_float, []),
     "rvo_set_option": (C.c_int, [C.c_char_p, C.c_int64]),

@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "lib", "librevers_o_b200.so")
-SOURCES = ["api.cu", "scan_tc.cu", "scan_tc2.cu", "select.cu", "prep_scan_small.cu", "mask_pool.cu", "mask_pool_tc.cu", "selfjoin.cu", "knn.cu"]
+SOURCES = ["api.cu", "scan_tc.cu", "scan_tc2.cu", "select.cu", "prep_scan_small.cu", "mask_pool.cu", "mask_pool_tc.cu", "selfjoin.cu", "knn.cu", "kmeans.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

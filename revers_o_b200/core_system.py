@@ -703,6 +703,47 @@ class SimpleReverso:
             results_text += f"   📍 First region: {it['members'][0]['filename']} {it['members'][0]['bbox']}\n\n"
         return results_text, items
 
+    def find_visual_themes(self, n_themes=20, max_themes=20, examples=5):
+        """New: what kinds of regions the loaded database holds, and how many of each — spherical k-means of its regions into
+        n_themes clusters on the GPU (`B200VectorDB.cluster`; fewer when the database holds fewer regions).  Returns (status
+        text, list of dict{size, images: distinct filenames, examples: [dict{filename, bbox, score}]}) for the `max_themes`
+        largest themes, largest first; the examples are the `examples` members nearest their theme's centre (highest score,
+        ties by the database's order)."""
+        if not self.vector_db or not self.current_database:
+            return "❌ No database loaded. Please create or load a database first.", []
+        print(f"🔍 Finding visual themes of {self.current_database} (n_themes={n_themes})")
+        try:
+            with self.vector_db._lock.read():
+                c = self.vector_db._coll(self.current_database)
+                if c.n == 0:
+                    return "❌ The database holds no regions", []
+                res = self.vector_db._cluster_rows(self.current_database, min(int(n_themes), c.n), 50, 0, None)
+                items = []
+                for t in range(min(max(int(max_themes), 0), len(res.sizes))):
+                    if res.sizes[t] == 0:
+                        break
+                    rows = np.flatnonzero(res.labels == t)
+                    best = rows[np.lexsort((rows, -res.scores[rows].astype(np.float64)))]
+                    pays = [c.payloads[int(r)] or {} for r in rows]
+                    ex = []
+                    for r in best[:max(int(examples), 0)]:
+                        pay = c.payloads[int(r)] or {}
+                        ex.append({"filename": pay.get("filename", "Unknown"), "bbox": pay.get("bbox"),
+                                   "score": float(res.scores[r])})
+                    items.append({"size": int(res.sizes[t]), "images": sorted({p.get("filename", "Unknown") for p in pays}),
+                                  "examples": ex})
+        except Exception as e:
+            return f"❌ Clustering error: {e}", []
+        results_text = f"🎯 Found {int((res.sizes > 0).sum())} visual themes in {c.n} regions, showing {len(items)}:\n\n"
+        for i, it in enumerate(items):
+            files = it["images"]
+            results_text += f"{i + 1}. {it['size']} regions in {len(files)} images: {', '.join(files[:5])}"
+            results_text += f" (+{len(files) - 5} more)\n" if len(files) > 5 else "\n"
+            if it["examples"]:
+                e = it["examples"][0]
+                results_text += f"   📍 Most typical region: {e['filename']} {e['bbox']} (Similarity: {e['score']:.3f})\n\n"
+        return results_text, items
+
     def visualize_detections(self, image, selected_region_index=None):
         """core_system.py:719-757 — rendering, out of scope; returns the image with region boxes drawn."""
         pil = self._to_pil(image).copy()

@@ -28,6 +28,12 @@ int launch_knn_intake(const uint16_t* qdb, long long row0, const int64_t* rows, 
 int launch_knn_exclude(const int64_t* ids, const float* scores, const int32_t* counts, int nq, int k, long long row0,
                        const int64_t* rows, long long q_id_offset, int64_t* out_ids, float* out_scores, int32_t* out_counts,
                        cudaStream_t stream);
+size_t kmeans_update_workspace_bytes(long long n, int C);
+int launch_kmeans_update(const uint16_t* db, long long row_lo, long long n, int d, int d_pad, const int64_t* ids, long long id_offset,
+                         int C, const int32_t* prev, int32_t* labels, int64_t* sums, int64_t* counts, int64_t* changed, void* ws,
+                         int sm_count, cudaStream_t stream);
+int launch_kmeans_finalize(const int64_t* sums, const int64_t* counts, int C, int d, float* out, int32_t* empty, int64_t* n_empty,
+                           cudaStream_t stream);
 static thread_local char g_err[512] = "";
 std::atomic<long long> g_launches{0};
 std::atomic<long long> g_chain_trace{0};
@@ -784,6 +790,60 @@ int rvo_knn_exclude_self(const int64_t* ids, const float* scores, const int32_t*
     if (rc) return rc;
     return launch_knn_exclude(ids, scores, counts, nq, k, q_row_lo, q_rows, q_id_offset, out_ids, out_scores, out_counts,
                               (cudaStream_t)stream);
+}
+
+// ---- spherical k-means update (kmeans.cu) ------------------------------------------------------------------------------
+
+size_t rvo_kmeans_update_workspace_bytes(int64_t n_rows, int32_t n_clusters) {
+    if (n_rows < 0 || n_rows >= (1ll << 31) || n_clusters < 1 || n_clusters > RVO_KMEANS_MAX_CLUSTERS) return 0;
+    return kmeans_update_workspace_bytes(n_rows, n_clusters);
+}
+
+int rvo_kmeans_update(const uint16_t* db, int64_t row_lo, int64_t row_hi, int32_t d, int64_t d_pad_in, const int64_t* ids,
+                      int64_t id_offset, int32_t n_clusters, const int32_t* prev_labels, int32_t* labels, int64_t* sums,
+                      int64_t* counts, int64_t* changed, void* workspace, size_t workspace_bytes, void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(db && ids && labels && sums && counts && changed && workspace, "kmeans update: null pointer");
+    RVO_REQUIRE(n_clusters >= 1 && n_clusters <= RVO_KMEANS_MAX_CLUSTERS, "kmeans update: n_clusters=%d outside 1..%d", n_clusters,
+                RVO_KMEANS_MAX_CLUSTERS);
+    RVO_REQUIRE(d > 0 && row_lo >= 0 && row_lo <= row_hi && row_hi - row_lo < (1ll << 31),
+                "kmeans update: bad shape d=%d rows [%lld,%lld) (fewer than 2^31 rows)", d, (long long)row_lo, (long long)row_hi);
+    RVO_REQUIRE(d_pad_in == (d + kBlockK - 1) / kBlockK * kBlockK, "kmeans update: d_pad must be d rounded up to 64");
+    RVO_REQUIRE(((uintptr_t)db & 15) == 0 && ((uintptr_t)sums & 7) == 0 && ((uintptr_t)counts & 7) == 0 &&
+                    ((uintptr_t)changed & 7) == 0 && ((uintptr_t)workspace & 255) == 0,
+                "kmeans update: alignment");
+    const long long n = row_hi - row_lo;
+    if (workspace_bytes < kmeans_update_workspace_bytes(n, n_clusters)) {
+        set_error("kmeans update workspace too small: %zu bytes given, %zu needed", workspace_bytes,
+                  kmeans_update_workspace_bytes(n, n_clusters));
+        return RVO_E_WORKSPACE;
+    }
+    int sm = 0;
+    int rc = select_device_of(db, &sm);
+    if (rc) return rc;
+    int ddev = -1, sdev = -1;
+    RVO_CUDA(cudaGetDevice(&ddev));
+    rc = select_device_of(sums, nullptr);
+    if (rc) return rc;
+    RVO_CUDA(cudaGetDevice(&sdev));
+    RVO_REQUIRE(ddev == sdev, "kmeans update: rows on device %d, sums on device %d", ddev, sdev);
+    return launch_kmeans_update(db, row_lo, n, d, (int)d_pad_in, ids, id_offset, n_clusters, prev_labels, labels, sums, counts,
+                                changed, workspace, sm, (cudaStream_t)stream);
+}
+
+int rvo_kmeans_finalize(const int64_t* sums, const int64_t* counts, int32_t n_clusters, int32_t d, float* scratch_f32,
+                        uint16_t* centroids, int32_t* out_empty, int64_t* n_empty, void* stream) {
+    DeviceGuard device_guard;
+    RVO_REQUIRE(sums && counts && scratch_f32 && centroids && out_empty && n_empty, "kmeans finalize: null pointer");
+    RVO_REQUIRE(n_clusters >= 1 && n_clusters <= RVO_KMEANS_MAX_CLUSTERS && d > 0, "kmeans finalize: n_clusters=%d d=%d",
+                n_clusters, d);
+    RVO_REQUIRE(((uintptr_t)centroids & 15) == 0 && ((uintptr_t)n_empty & 7) == 0, "kmeans finalize: alignment");
+    int rc = select_device_of(sums, nullptr);
+    if (rc) return rc;
+    rc = launch_kmeans_finalize(sums, counts, n_clusters, d, scratch_f32, out_empty, n_empty, (cudaStream_t)stream);
+    if (rc) return rc;
+    const long long d_pad = (d + kBlockK - 1) / kBlockK * kBlockK;
+    return launch_normalize_rows(scratch_f32, n_clusters, d, d, centroids, d_pad, 0, nullptr, d, (cudaStream_t)stream);
 }
 
 // ---- peer-memory exchange (DESIGN.md §5) ------------------------------------------------------------------------------

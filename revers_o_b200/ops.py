@@ -596,3 +596,57 @@ def merge_topk(ids: torch.Tensor, scores: torch.Tensor, counts: torch.Tensor, k:
     check(_lib.load().rvo_merge_topk(_ptr(ids), _ptr(scores), _ptr(counts), G, nq, k, _ptr(oi), _ptr(os_), _ptr(oc),
                                      _stream(dev)), "rvo_merge_topk")
     return oi, os_, oc
+
+
+def kmeans_update(db: torch.Tensor, row_lo: int, row_hi: int, d: int, ids: torch.Tensor, n_clusters: int, prev: torch.Tensor | None,
+                  labels: torch.Tensor, sums: torch.Tensor, counts: torch.Tensor, changed: torch.Tensor, id_offset: int = 0) -> None:
+    """rvo_kmeans_update: the update step of spherical k-means for rows [row_lo, row_hi) of the tiled storage `db`, assigned by
+    `ids` (int64 [n] or [n, 1], the k = 1 lists of `knn_join` against the centroids; cluster = id - id_offset).  Writes int32
+    `labels` [n] and ADDS to `sums` (int64 [n_clusters, d]: each member's bf16 components as rint(x * 2^31), exact and
+    order-independent), `counts` (int64 [n_clusters]) and `changed` (int64 [1]: labels differing from `prev`, all n when prev is
+    None).  Async on the current stream of db's device."""
+    require_cuda(db, "db")
+    assert db.dtype == torch.bfloat16 and db.dim() == 4 and db.is_contiguous() and db.shape[1] * TILE_COLS == d_pad_of(d)
+    n = int(row_hi) - int(row_lo)
+    assert row_hi <= db_capacity(db) and ids.dtype == torch.int64 and ids.is_contiguous() and ids.numel() == n
+    assert labels.dtype == torch.int32 and labels.is_contiguous() and labels.numel() == n
+    assert prev is None or (prev.dtype == torch.int32 and prev.is_contiguous() and prev.numel() == n)
+    assert sums.dtype == counts.dtype == changed.dtype == torch.int64 and sums.shape == (n_clusters, d) and sums.is_contiguous()
+    assert counts.shape == (n_clusters,) and changed.numel() >= 1
+    dev = db.device
+    lib = _lib.load()
+    nbytes = lib.rvo_kmeans_update_workspace_bytes(n, int(n_clusters))
+    if nbytes == 0:
+        raise RvoError(f"k-means update of {n} rows into {n_clusters} clusters: needs fewer than 2^31 rows and 1 to "
+                       f"{_lib.RVO_KMEANS_MAX_CLUSTERS} clusters")
+    ws = workspace(dev, nbytes, "kmeans")
+    check(lib.rvo_kmeans_update(_ptr(db), int(row_lo), int(row_hi), d, d_pad_of(d), _ptr(ids), int(id_offset), int(n_clusters),
+                                _ptr(prev), _ptr(labels), _ptr(sums), _ptr(counts), _ptr(changed), _ptr(ws), nbytes, _stream(dev)),
+          "rvo_kmeans_update")
+
+
+def kmeans_finalize(sums: torch.Tensor, counts: torch.Tensor, d: int, centroids: torch.Tensor, empty: torch.Tensor,
+                    n_empty: torch.Tensor) -> None:
+    """rvo_kmeans_finalize: new centroids from the (reduced) integer sums, normalised and rounded into rows [0, C) of the tiled
+    storage `centroids` as `normalize_rows` does; `empty` (int32 [C]) flags the clusters with no member or an all-zero sum, and
+    their number is ADDED to `n_empty` (int64 [1]).  Async on the current stream of the sums' device."""
+    require_cuda(sums, "sums")
+    C = sums.shape[0]
+    assert sums.dtype == counts.dtype == n_empty.dtype == torch.int64 and sums.shape == (C, d) and counts.shape == (C,)
+    assert centroids.dtype == torch.bfloat16 and centroids.is_contiguous() and C <= db_capacity(centroids)
+    assert centroids.shape[1] * TILE_COLS == d_pad_of(d) and empty.dtype == torch.int32 and empty.numel() == C
+    for t in (counts, centroids, empty, n_empty):
+        assert t.device == sums.device
+    scratch = workspace(sums.device, C * d * 4, "kmeans_f32")
+    check(_lib.load().rvo_kmeans_finalize(_ptr(sums), _ptr(counts), C, d, _ptr(scratch), _ptr(centroids), _ptr(empty), _ptr(n_empty),
+                                          _stream(sums.device)), "rvo_kmeans_finalize")
+
+
+def kmeans_exact(db: torch.Tensor, n_rows: int, d: int, centroids: torch.Tensor, n_clusters: int, max_iter: int = 50,
+                 id_offset: int = 0):
+    """Spherical k-means of the first n_rows rows of the tiled storage `db`, started from rows [0, n_clusters) of the tiled
+    centroid storage `centroids` (on db's device; it is not modified).  The loop of `sharded.kmeans_sharded` on one shard:
+    assignment `knn_exact(db, 0, n, id_offset, centroids, C, d, 1, None, 0, False)`, integer update, re-seeding of empty
+    clusters, until an assignment equals the previous one or max_iter updates have run.  Returns `sharded.KMeansResult`."""
+    from .sharded import kmeans_sharded
+    return kmeans_sharded([(db, int(n_rows), int(id_offset))], d, centroids, n_clusters, max_iter)

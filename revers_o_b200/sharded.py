@@ -15,7 +15,9 @@ query blocks.  So is the join between two such collections (B200VectorDB.join_co
 `crossjoin_sharded`, run by the same device loop, and the duplicate groups of a row-sharded collection
 (B200VectorDB.find_duplicate_groups): `components_sharded`, the self-join's items unioned into one forest per device.  The
 k-nearest-neighbour join of two such collections, or of one with itself (B200VectorDB.knn_join), is `knn_plan` and `knn_sharded`:
-per-shard lists merged by K3 on the left shard's device, sharing the staging code (`_Staging`) of the joins.
+per-shard lists merged by K3 on the left shard's device, sharing the staging code (`_Staging`) of the joins.  Spherical k-means of
+such a collection (B200VectorDB.cluster) is `kmeans_sharded`: every shard assigned and summed on its own device, the integer sums
+added on the first device.
 """
 from __future__ import annotations
 
@@ -482,6 +484,138 @@ def _knn_overflow(left_shard, off: int, bad: torch.Tensor, right: list, d: int, 
         idx = bad + off
         for dst, src in zip(out, res):
             dst[idx] = src.cpu()
+
+
+class KMeansResult(NamedTuple):
+    """Spherical k-means in the clusters' own numbering.  labels int32 [N] and scores float32 [N] (host, global row order):
+    every row's assignment to `centroids`; centroids: the tiled bf16 storage of the C centroids (on the first device);
+    sizes int64 [C] (host): members per cluster; iterations: updates run; converged: the last assignment equals the previous."""
+    labels: np.ndarray
+    scores: np.ndarray
+    centroids: torch.Tensor
+    sizes: np.ndarray
+    iterations: int
+    converged: bool
+
+
+def gather_rows(shards: list, rows, d: int, device: torch.device) -> torch.Tensor:
+    """The stored bf16 rows `rows` (global rows of shards [(tiled storage, rows, first global row)]) copied bit for bit into
+    rows [0, len(rows)) of a new tiled storage on `device`."""
+    rows = torch.as_tensor(np.asarray(rows, dtype=np.int64))
+    out = ops.db_alloc(max(len(rows), 1), d, device)
+    dst = torch.arange(len(rows), dtype=torch.int64)
+    for v, n, r0 in shards:
+        sel = ((rows >= r0) & (rows < r0 + n)).nonzero().flatten()
+        if sel.numel():
+            lr = (rows[sel] - r0).to(v.device)
+            o = dst[sel].to(device)
+            out[o // ops.TILE_ROWS, :, o % ops.TILE_ROWS, :] = v[lr // ops.TILE_ROWS, :, lr % ops.TILE_ROWS, :].to(device)
+    return out
+
+
+def reseed_rows(scores: list, row0s: list, n_empty: int) -> list:
+    """The rows that re-seed `n_empty` empty clusters: the rows with the lowest assignment scores, ties by the lower row, in that
+    order (cluster j of the empty ones, in index order, takes entry j).  scores: one 1-d tensor per shard, the scores of its rows
+    in row order; row0s: each shard's first global row.  Each shard offers its n_empty lowest, so only those are compared."""
+    dev = scores[0].device
+    cand_s, cand_r = [], []
+    for sc, r0 in zip(scores, row0s):
+        o = torch.sort(sc, stable=True).indices[:n_empty]             # ascending, equal scores in row order
+        cand_s.append(sc[o].to(dev))
+        cand_r.append((o + int(r0)).to(dev))
+    s, r = torch.cat(cand_s), torch.cat(cand_r)
+    o = torch.argsort(r)
+    s, r = s[o], r[o]
+    return r[torch.sort(s, stable=True).indices[:n_empty]].tolist()
+
+
+def kmeans_sharded(shards: list, d: int, centroids: torch.Tensor, n_clusters: int, max_iter: int = 50) -> KMeansResult:
+    """Spherical k-means of a collection row-sharded over the devices of one process; no row moves.  shards: [(tiled storage,
+    rows, first global row)] in row order, covering the global rows [0, N) with N < 2^31; `centroids`: tiled storage holding the
+    C = n_clusters initial centroids on the first device (not modified).
+
+    Assign, then, while fewer than max_iter updates have run, update and assign again; stop at the first assignment equal to
+    the previous one (the centroids are then a fixed point).  Each iteration:
+      - the centroid buffer (2 C d_pad bytes) is peer-copied from the first device to every other shard device;
+      - every shard runs `ops.knn_join` (k = 1) of its rows against it on its own device, all enqueued before the overflow
+        check, and rows the fused path flags go through the exact fp32 routes (`ops.knn_fp32`): `ops.knn_exact`'s protocol;
+      - `ops.kmeans_update` turns each shard's assignment into labels and adds its members to its device's int64 sums and
+        counts; the other devices' sums, counts and change counts are peer-copied to the first device and added there.  The
+        sums are integers, so the result does not depend on the shard layout;
+      - `ops.kmeans_finalize` normalises the sums into the next centroid buffer, and one host synchronisation reads the
+        change count and the number of empty clusters;
+      - each empty cluster (no member, or an all-zero sum), in index order, takes the stored row `reseed_rows` gives.
+    Memory per device: sums 8 C d and counts 8 C bytes, the centroid buffer(s), the assignment (21 bytes per row of its shards)
+    and the workspaces of `knn_join` and `kmeans_update`."""
+    C, max_iter = int(n_clusters), int(max_iter)
+    n_total = sum(int(n) for _, n, _ in shards)
+    if not 0 < n_total < (1 << 31):
+        raise _lib.RvoError(f"k-means needs 1 to 2^31 - 1 rows, got {n_total}")
+    if not 1 <= C <= min(n_total, _lib.RVO_KMEANS_MAX_CLUSTERS):
+        raise _lib.RvoError(f"k-means: n_clusters={C} outside 1..{min(n_total, _lib.RVO_KMEANS_MAX_CLUSTERS)}")
+    if max_iter < 0:
+        raise _lib.RvoError(f"k-means: max_iter={max_iter} < 0")
+    home = centroids.device
+    devs = list(dict.fromkeys([home] + [v.device for v, _, _ in shards]))
+    acc = {dv: (torch.zeros((C, d), dtype=torch.int64, device=dv), torch.zeros((C,), dtype=torch.int64, device=dv),
+                torch.zeros((2,), dtype=torch.int64, device=dv)) for dv in devs}          # sums, counts, (changed, empty)
+    cent = [ops.db_alloc(C, d, home), ops.db_alloc(C, d, home)]
+    cent[0].copy_(centroids[: cent[0].shape[0]])
+    local = {dv: ops.db_alloc(C, d, dv) for dv in devs if dv != home}
+    empty = torch.zeros((C,), dtype=torch.int32, device=home)
+    assign = [(torch.empty((n, 1), dtype=torch.int64, device=v.device), torch.empty((n, 1), dtype=torch.float32, device=v.device),
+               torch.empty((n,), dtype=torch.int32, device=v.device)) for v, n, _ in shards]
+    labels = [[torch.empty((n,), dtype=torch.int32, device=v.device) for v, n, _ in shards] for _ in range(2)]
+    it, cur, converged = 0, 0, False
+    while True:
+        for dv, buf in local.items():
+            with torch.cuda.device(dv):
+                buf.copy_(cent[0], non_blocking=True)          # a peer copy, after the home stream's finalise, before the joins
+        for (v, n, r0), out in zip(shards, assign):
+            with torch.cuda.device(v.device):
+                ops.knn_join(v, 0, n, r0, local.get(v.device, cent[0]), C, d, 1, None, 0, False, out=out)
+        for (v, n, r0), (ids, sc, cnt) in zip(shards, assign):
+            bad = (cnt < 0).nonzero().flatten()                # host sync; pathological inputs only take the branch
+            if bad.numel() and ops.d_pad_of(d) > 2048:
+                raise _lib.RvoError(f"k-means: rows {(bad + r0).tolist()[:20]} overflowed the candidate lists and rows of {d} "
+                                    "dims (> 2048) have no exact fp32 route")
+            if bad.numel():
+                with torch.cuda.device(v.device):
+                    ids[bad], sc[bad], cnt[bad] = ops.knn_fp32(v, bad, r0, local.get(v.device, cent[0]), C, d, 1, None, 0, False)
+        for g, ((v, n, _), (ids, _, _)) in enumerate(zip(shards, assign)):
+            sums, counts, stats = acc[v.device]
+            with torch.cuda.device(v.device):
+                ops.kmeans_update(v, 0, n, d, ids, C, labels[1 - cur][g] if it else None, labels[cur][g], sums, counts, stats[:1])
+        sums, counts, stats = acc[home]
+        with torch.cuda.device(home):
+            for dv in devs[1:]:                                  # integer additions: any order gives the same sums
+                sums += acc[dv][0].to(home)
+                counts += acc[dv][1].to(home)
+                stats[:1] += acc[dv][2][:1].to(home)
+            if it < max_iter:
+                ops.kmeans_finalize(sums, counts, d, cent[1], empty, stats[1:])
+        changed, n_empty = stats.tolist()
+        if it and changed == 0:
+            converged = True
+            break
+        if it == max_iter:
+            break
+        if n_empty:
+            which = empty.nonzero().flatten().tolist()
+            rows = reseed_rows([a[1].view(-1) for a in assign], [r0 for _, _, r0 in shards], len(which))
+            seeds = gather_rows(shards, rows, d, home)
+            w = torch.tensor(which, dtype=torch.int64, device=home)
+            j = torch.arange(len(which), dtype=torch.int64, device=home)
+            cent[1][w // ops.TILE_ROWS, :, w % ops.TILE_ROWS, :] = seeds[j // ops.TILE_ROWS, :, j % ops.TILE_ROWS, :]
+        cent.reverse()
+        cur = 1 - cur
+        it += 1
+        for a in acc.values():
+            for t in a:
+                t.zero_()
+    lab = np.concatenate([x.cpu().numpy() for x in labels[cur]])
+    sc = np.concatenate([a[1].view(-1).cpu().numpy() for a in assign])
+    return KMeansResult(lab, sc, cent[0], acc[home][1].cpu().numpy(), it, converged)
 
 
 def _join_runs(its: list[JoinItem], shards: list, dv: int) -> list[JoinItem]:

@@ -9,7 +9,9 @@ It duck-types exactly the five qdrant-client methods core_system.py uses (SURVEY
 plus the batched entry point `search_batch` (new; reduces to `search` row by row, SURVEY.md F7), and two threshold joins
 (new): `find_near_duplicates` (every pair within one collection at cos >= threshold) and `join_collections` (every pair across
 two collections, possibly of two B200VectorDB instances: which regions of one archive also appear in another), and the groups
-of the first (new): `find_duplicate_groups` (the connected components of those pairs, unioned on the GPU, no pair stored).
+of the first (new): `find_duplicate_groups` (the connected components of those pairs, unioned on the GPU, no pair stored),
+`knn_join` (every point's k best matches) and `cluster` (new: spherical k-means of a collection, integer-exact updates, the
+same result on any shard layout).
 
 Vectors live on the GPU(s) as L2-normalised bf16 rows in the TILED storage of include/revers_o_b200.h
 ([row/128][col/64][128][64]: one contiguous 16 KiB TMA box per tile; the DB is DEFINED as its bf16 values).  All arithmetic
@@ -813,6 +815,49 @@ class B200VectorDB:
                            f"and rows of {a.dim} dims (> 2048) have no exact fp32 route")
         return rows, scores, counts
 
+    def cluster(self, collection_name: str, n_clusters: int, max_iter: int = 50, seed: int = 0, init=None) -> Clusters:
+        """Spherical k-means: "what kinds of things are in this collection, and how much of each?".  Partitions the stored
+        points into n_clusters clusters around centre directions, computed on the GPU(s) where the collection lives
+        (`sharded.kmeans_sharded`; no row moves).
+
+        - A centroid is stored like a point: L2-normalised, rounded to bf16.  A point's score against a centroid is the fp32
+          dot of the two stored bf16 vectors, and its label is the centroid with the highest score, ties to the lower index
+          (`knn_join` with k = 1 against the centroids).
+        - Update: a cluster's new centroid is the normalised sum of its members, rounded to bf16.  The sum is accumulated in
+          integer fixed point (each component as an integer multiple of 2^-31), so it is exact in any order and the result is
+          bit-identical on any shard layout.
+        - Initial centroids: `init` [n_clusters, dim] (normalised and rounded as `upsert` does), or by default the stored points
+          of rows `numpy.random.default_rng(seed).choice(n, n_clusters, replace=False)`, copied bit for bit.
+        - A cluster left with no member (or an all-zero sum) is re-seeded: in index order, each takes the point with the lowest
+          score in the assignment not already taken, ties by the lower row.
+        - Assign; then, while fewer than max_iter updates have run, update and assign again; stop at the first assignment equal
+          to the previous one (`converged`).  max_iter = 0 is the assignment to the initial centroids.
+        Returns `Clusters` with labels and scores of the last assignment, to the returned centroids, and the clusters renumbered
+        by `cluster_order`: largest first, equal sizes by their first member row, empty ones last.  The collection stays
+        read-locked for the call."""
+        with self._lock.read():
+            return self._cluster_rows(collection_name, n_clusters, max_iter, seed, init)
+
+    def _cluster_rows(self, collection_name: str, n_clusters: int, max_iter: int, seed: int, init) -> Clusters:
+        """`cluster`; the caller holds the read lock."""
+        from .sharded import gather_rows, kmeans_sharded
+        c = self._coll(collection_name)
+        init = check_cluster_args(c.n, c.dim, n_clusters, max_iter, init)
+        C = int(n_clusters)
+        shards = [(s.vectors, s.n, s.row0) for s in c.shards if s.n]
+        home = shards[0][0].device
+        if init is None:
+            cent = gather_rows(shards, np.random.default_rng(seed).choice(c.n, C, replace=False), c.dim, home)
+        else:
+            cent = ops.db_alloc(C, c.dim, home)
+            with torch.cuda.device(home):
+                ops.normalize_rows(torch.from_numpy(init).to(home), db=cent, row0=0)
+        r = kmeans_sharded(shards, c.dim, cent, C, max_iter)
+        labels, order, sizes = cluster_order(r.labels, C)
+        cf = ops.untile_rows(r.centroids, C, c.dim).float().cpu().numpy()
+        return Clusters(labels=labels, scores=r.scores, centroids=cf[order], sizes=sizes, iterations=r.iterations,
+                        converged=r.converged)
+
     def count(self, collection_name: str) -> int:
         return self._coll(collection_name).n
 
@@ -1118,6 +1163,60 @@ def mutual_best(rows_ab, counts_ab, rows_ba, counts_ba, scores_ab):
     s = scores_ab[a, 0] if a.size else np.zeros(0, np.float32)
     o = np.lexsort((b, a, -s.astype(np.float64)))
     return np.stack([a[o], b[o]], 1).astype(np.int64).reshape(-1, 2), s[o].astype(np.float32)
+
+
+@dataclass
+class Clusters:
+    """`B200VectorDB.cluster`'s result, clusters numbered by `cluster_order`.  labels int32 [n] and scores float32 [n] in row
+    order: each point's cluster and its score against that cluster's centroid; centroids float32 [C, dim]: the bf16 values of
+    the centroids; sizes int64 [C]: members per cluster; iterations: updates run; converged: the last assignment equals the
+    one before it."""
+    labels: np.ndarray
+    scores: np.ndarray
+    centroids: np.ndarray
+    sizes: np.ndarray
+    iterations: int
+    converged: bool
+
+
+def check_cluster_args(n: int, dim: int, n_clusters, max_iter, init):
+    """`B200VectorDB.cluster`'s argument checks for a collection of n points of `dim` dimensions; raises RvoError.  Returns
+    `init` as a float32 array [n_clusters, dim], or None."""
+    if n == 0:
+        raise RvoError("cluster: the collection is empty")
+    if n >= (1 << 31):
+        raise RvoError(f"cluster: {n} points; k-means takes fewer than 2^31")
+    hi = min(n, _lib.RVO_KMEANS_MAX_CLUSTERS)
+    if isinstance(n_clusters, bool) or int(n_clusters) != n_clusters or not 1 <= int(n_clusters) <= hi:
+        raise RvoError(f"cluster: n_clusters={n_clusters} outside 1..{hi}")
+    if isinstance(max_iter, bool) or int(max_iter) != max_iter or int(max_iter) < 0:
+        raise RvoError(f"cluster: max_iter={max_iter} must be an integer >= 0")
+    if init is None:
+        return None
+    x = (init.detach().float().cpu().numpy() if isinstance(init, torch.Tensor) else np.asarray(init, dtype=np.float32))
+    x = np.ascontiguousarray(x, dtype=np.float32)
+    if x.shape != (int(n_clusters), dim):
+        raise RvoError(f"cluster: init has shape {x.shape}, expected ({int(n_clusters)}, {dim})")
+    bad = np.flatnonzero(~np.isfinite(x).all(1) | ~(np.abs(x) > 0).any(1))
+    if bad.size:
+        raise RvoError(f"cluster: init rows {bad[:20].tolist()} are zero or not finite")
+    return x
+
+
+def cluster_order(labels, n_clusters: int):
+    """Renumber clusters largest first; equal sizes by their first member row; empty clusters last, in index order.  labels:
+    int [n] in 0..n_clusters-1.  Returns (labels int32 [n] renumbered, order int64 [C]: the old index of each new cluster,
+    sizes int64 [C] in the new order)."""
+    labels = np.asarray(labels, dtype=np.int64)
+    C = int(n_clusters)
+    sizes = np.bincount(labels, minlength=C).astype(np.int64)
+    first = np.arange(C, dtype=np.int64) + labels.size          # empty clusters: after every row, in index order
+    u, idx = np.unique(labels, return_index=True)
+    first[u] = idx
+    order = np.lexsort((first, -sizes))
+    new = np.empty(C, np.int64)
+    new[order] = np.arange(C)
+    return new[labels].astype(np.int32), order.astype(np.int64), sizes[order]
 
 
 def _copy_blocks_to_device(view: np.ndarray, dst: torch.Tensor, chunk_blocks: int = 4096) -> None:
